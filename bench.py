@@ -4,10 +4,11 @@ config C5): 10^6 aircraft-scenarios per GPU x 10^4 RK4 steps, dt = 0.01 s, rando
 DFFF controller, log decimated x100.  One bench "step" = one full sweep.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # the CUDA engine
+    python bench.py ... --dump-outputs bench_outputs               # also write the last timed sweep's results as .npy files
     python bench.py --impl reference ...                           # the CPU arm (C port of the oracle, all host threads)
 
-Prints ONE JSON line (contract in the task statement: value = device-resident throughput, e2e = through the public
-host-buffer API with H2D/D2H inside the timed region, roofline, cpu_baseline, clocks, gpu_launches)."""
+Prints ONE JSON line (value = device-resident throughput, e2e = through the public host-buffer API with H2D/D2H inside
+the timed region, roofline, cpu_baseline, clocks, gpu_launches)."""
 import argparse
 import json
 import os
@@ -143,6 +144,31 @@ def _timed(fn, reps, warm=3):
         fn()
     e1.record(); e1.synchronize()
     return e0.elapsed_time(e1) * 1e-3 / reps
+
+
+DUMP_SCENARIOS = 4096
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, mc, seed):
+    """Writes what the timed sweep (MonteCarloRollout.run_device) left in HBM, under the names MonteCarloRollout.run()
+    returns them by, as float64 .npy files: the population statistics whole, every per-scenario array for the same sample
+    of at most DUMP_SCENARIOS scenarios (sorted indices drawn from `seed`, so equal arguments give an equal sample) in
+    run()'s layout, at most DUMP_BYTES in all.  Two builds run with the same arguments can then be compared file by file;
+    pop_sum_sq_err is summed with one atomicAdd per warp, so it may differ in its last bits from run to run."""
+    import torch
+    per_scenario = 8 * (mc.n_rows * (5 + (2 if mc.d_Ulog is not None else 0)) + 5 + 3)
+    S = min(mc.B, DUMP_SCENARIOS, DUMP_BYTES // per_scenario)
+    if S < 1:
+        raise SystemExit(f"--dump-outputs: the log of one scenario ({per_scenario} bytes) exceeds {DUMP_BYTES} bytes; raise --log-every")
+    idx = torch.from_numpy(np.sort(np.random.default_rng(seed).choice(mc.B, S, replace=False))).to(mc.d_Xf.device)
+    arrays = {"X_final": mc.d_Xf[:, idx].T, "sum_sq_err": mc.d_ss[idx], "max_err": mc.d_mx[idx], "flags": mc.d_flags[idx],
+              "pop_sum_sq_err": mc.d_pop[:1], "pop_max_err": mc.d_pop[1:], "X_log": mc.d_Xlog[:, :, idx]}
+    if mc.d_Ulog is not None:
+        arrays["U_log"] = mc.d_Ulog[:, :, idx]
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.to(torch.float64).cpu().numpy())
 
 
 C4 = dict(n_ac=16, N=500, h=0.02)
@@ -502,7 +528,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--core-only", action="store_true", help="skip the single-GPU extras (planner solves, tracker, pursuit, CPU figures)")
     ap.add_argument("--seed", type=int, default=12345)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed sweep (a fixed sample of the "
+                                                          "scenarios, at most 64 MB) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "d2dx":
+        ap.error("--dump-outputs applies to the CUDA engine (--impl d2dx)")
     args.warmup = max(args.warmup, 0)
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     config = {"workload": "C5 Monte-Carlo sweep: DFFF closed loop on random circles", "scenarios_per_gpu": args.scenarios,
@@ -603,6 +635,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     pop = reduce_population_stats(mc.d_pop.clone())
     flags_bad = int(mc.d_flags.ne(0).sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, mc, args.seed)
     ms_per_step = ms_total / max(args.steps, 1)
     total_steps = float(B) * T_steps * world
     value = total_steps / (ms_per_step * 1e-3)
