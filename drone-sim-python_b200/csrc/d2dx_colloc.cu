@@ -2,8 +2,8 @@
 // sparse Jacobian, the planner cost and its gradient, over problems x aircraft x nodes.
 // Three kernels share the per-(aircraft, node) work of d2dx_colloc_dev.cuh:
 //   colloc_kernel<false>   residual + Jacobian + input cost + gradient: the lean HBM-bound path (64 registers);
-//   colloc_kernel<true>    + obstacles, the reference's (0,1)-only collision term, ordered all-pairs loops (aircraft shards,
-//                          very large n_ac);
+//   colloc_kernel<true>    + obstacles, the reference's (0,1)-only collision term, ordered all-pairs loops (all-pairs
+//                          problems past colloc_pairs_kernel's shared-memory budget or 32-bit output offsets);
 //   colloc_pairs_kernel    all-pairs collision of one unsharded problem: one warp = one aircraft x 32 nodes, every unordered
 //                          pair evaluated once, its exponential handed to the partner through a write-once shared-memory slot.
 // Every global load and store is coalesced along the node index.
@@ -45,12 +45,13 @@ __device__ __forceinline__ void cost_finish(const CollocArgs& a, int prob, int p
   }
 }
 
-// EXTRA = obstacle and / or collision terms present (exp, shared-memory partner loop); the plain instantiation is the lean
-// HBM-bound path (residual + Jacobian + input cost + gradient) and is held to 64 registers for occupancy.
+// EXTRA = obstacle and / or collision terms present (exp, shared-memory partner loop): obstacles, the (0,1) pair mode and
+// all-pairs problems colloc_pairs_kernel does not take.  The plain instantiation is the lean HBM-bound path (residual +
+// Jacobian + input cost + gradient) and is held to 64 registers for occupancy.
 // One thread = one (aircraft, node); a block covers a tile of TN nodes for APP aircraft per pass.
 template <bool EXTRA>
 __global__ void __launch_bounds__(kCollocThreads, EXTRA ? 5 : 8) colloc_kernel(const __grid_constant__ CollocArgs a) {
-  extern __shared__ double spos[];                 // [n_total][2][TN] positions of every aircraft on this tile
+  extern __shared__ double spos[];                 // [n_ac][2][TN] positions of every aircraft on this tile
   __shared__ double sred[kCollocThreads / 32][4];
   const d2dx_colloc_problem& P = a.p;
   const int N = P.N, n_ac = P.n_ac, TN = a.TN;
@@ -60,17 +61,14 @@ __global__ void __launch_bounds__(kCollocThreads, EXTRA ? 5 : 8) colloc_kernel(c
   const int i = tile * TN + il;
   const double* fr = a.free_ + (size_t)prob * a.n_free;
   const bool want_cg = (a.what & (D2DX_EVAL_COST | D2DX_EVAL_GRAD)) != 0;
-  const bool use_col = EXTRA && want_cg && enabled(P.kcol) && a.n_total > 1;
+  const bool use_col = EXTRA && want_cg && enabled(P.kcol) && n_ac > 1;
   const bool use_obs = EXTRA && want_cg && enabled(P.kobs) && P.n_obs > 0;
 
   if (use_col) {                                   // stage the tile's positions of ALL aircraft
-    for (int idx = tid; idx < a.n_total * TN; idx += kCollocThreads) {
+    for (int idx = tid; idx < n_ac * TN; idx += kCollocThreads) {
       const int g = idx / TN, ii = idx - g * TN, node = tile * TN + ii;
       double x = 0.0, y = 0.0;
-      if (node < N) {
-        if (a.pos_all) { x = a.pos_all[((size_t)g * 2) * N + node]; y = a.pos_all[((size_t)g * 2 + 1) * N + node]; }
-        else { x = fr[(3 * g) * N + node]; y = fr[(3 * g + 1) * N + node]; }
-      }
+      if (node < N) { x = fr[(3 * g) * N + node]; y = fr[(3 * g + 1) * N + node]; }
       spos[(g * 2) * TN + ii] = x; spos[(g * 2 + 1) * TN + ii] = y;
     }
     __syncthreads();
@@ -86,19 +84,18 @@ __global__ void __launch_bounds__(kCollocThreads, EXTRA ? 5 : 8) colloc_kernel(c
     const double x = fr[ox], y = fr[ox + N];
     double gx = 0.0, gy = 0.0;
     if (EXTRA && want_cg) {
-      const int g_glob = a.a_lo + a_l;
-      if (use_obs && g_glob == 0) obstacle_terms(P, sN, x, y, s_obs, gx, gy);   // CostObstacle acts on aircraft 0 only (multiopty_utils.py:74)
+      if (use_obs && a_l == 0) obstacle_terms(P, sN, x, y, s_obs, gx, gy);   // CostObstacle acts on aircraft 0 only (multiopty_utils.py:74)
       if (use_col) {                               // CostCollision (multiopty_utils.py:120-153), partners from shared memory
         const double cw = a.cw;
-        const int b_lo = P.col_all_pairs ? 0 : (g_glob == 0 ? 1 : 0);
-        const int b_hi = P.col_all_pairs ? a.n_total : (g_glob == 0 ? 2 : (g_glob == 1 ? 1 : 0));
+        const int b_lo = P.col_all_pairs ? 0 : (a_l == 0 ? 1 : 0);
+        const int b_hi = P.col_all_pairs ? n_ac : (a_l == 0 ? 2 : (a_l == 1 ? 1 : 0));
         const double* sp = spos + il;
         for (int b = b_lo; b < b_hi; ++b) {
-          if (b == g_glob) continue;
+          if (b == a_l) continue;
           const double dx = x - sp[(b * 2) * TN], dy = y - sp[(b * 2 + 1) * TN];
           const double ux = dx * col_kr, uy = dy * col_kr;
           const double es = fm::exp_neg(-(ux * ux + uy * uy));
-          if (g_glob < b) s_col += es;             // each pair counted once, at its lower-index member
+          if (a_l < b) s_col += es;                // each pair counted once, at its lower-index member
           const double w = cw * es;
           gx = fma(w, dx, gx); gy = fma(w, dy, gy);
         }
@@ -259,7 +256,7 @@ __global__ void __launch_bounds__(kPairWarps * 32, REGS ? 4 : 3) colloc_pairs_ke
       gx = fma(wgt, xa - pb[0], gx); gy = fma(wgt, ya - pb[R], gy);
     }
     }
-    if (valid) {                                   // 32-bit flat output indices: launch_eval checks
+    if (valid) {                                   // 32-bit flat output indices: d2dx_colloc_eval checks
       const NodeOff o = colloc_offsets(P, a_l, i);
       const NodeIn in = {fr[o.ox + 2 * N], fr[o.ophi], fr[o.ov], pa[-1], pa[R - 1], i >= 1 ? fr[o.ox + 2 * N - 1] : 0.0};
       colloc_node_in<true, true>(a, prob, a_l, i, xa, ya, in, o, gx, gy, true, s_v, s_phi);
@@ -375,15 +372,6 @@ __global__ void colloc_init_dense_kernel(long nnz, int n_inst, int n_prob, doubl
     jac[idx] = (idx % nnz) >= nnz - n_inst ? 1.0 : 0.0;
 }
 
-__global__ void pack_positions_kernel(int n_ac, int N, const double* __restrict__ fr, double* __restrict__ pos) {
-  const long total = (long)n_ac * 2 * N;
-  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
-    const int g = (int)(idx / (2L * N));
-    const long rem = idx - (long)g * 2 * N;        // c*N + node ; x,y slices are adjacent in the planner layout
-    pos[idx] = fr[(size_t)(3 * g) * N + rem];
-  }
-}
-
 // CostBank with use_mean = False (d2d/opty_utils.py:68-82): cost = obj_scale max_i phi_i^2; gradient = one entry
 // obj_scale 2 phi_i at i = np.argmax(phi^2) (first maximum), zeros elsewhere.  One block per problem.
 __global__ void __launch_bounds__(256) bank_max_kernel(int n_free, int off_phi, int N, double obj_scale, const double* __restrict__ free_,
@@ -457,67 +445,6 @@ static int check_problem(const d2dx_colloc_problem* p, const char* who) {
   return D2DX_OK;
 }
 
-static int launch_eval(d2dx_handle* h, const d2dx_colloc_problem* p, int n_prob, int n_total, int a_lo, const double* free_,
-                       const double* pos_all, int layout, uint32_t what, double* residual, double* jac, double* cost,
-                       double* grad, double* scratch, void* stream, const char* who) {
-  if (int rc = check_problem(p, who)) return rc;
-  D2DX_CHECK_ARG(h && free_ && n_prob >= 1 && n_prob <= 65536, "%s: n_prob=%d (1..65536 per call)", who, n_prob);
-  D2DX_CHECK_ARG(layout == D2DX_JAC_COMPACT || layout == D2DX_JAC_OPTY_DENSE, "%s: unknown Jacobian layout %d", who, layout);
-  D2DX_CHECK_ARG(!(what & D2DX_EVAL_RESIDUAL) || residual, "%s: residual requested but NULL", who);
-  D2DX_CHECK_ARG(!(what & D2DX_EVAL_JAC) || jac, "%s: jacobian requested but NULL", who);
-  D2DX_CHECK_ARG(!(what & D2DX_EVAL_COST) || (cost && scratch), "%s: cost requested but cost/scratch NULL", who);
-  D2DX_CHECK_ARG(!(what & D2DX_EVAL_GRAD) || grad, "%s: gradient requested but NULL", who);
-  D2DX_CHECK_ARG(5L * p->n_ac * p->N < (1L << 31), "%s: 5 n_ac N = %ld does not fit 32-bit offsets", who, 5L * p->n_ac * p->N);
-  CollocArgs a;
-  a.p = *p; a.n_prob = n_prob; a.layout = layout; a.what = what; a.free_ = free_;
-  a.res = residual; a.jac = jac; a.cost = cost; a.grad = grad; a.scratch = scratch;
-  a.n_total = n_total; a.a_lo = a_lo; a.pos_all = pos_all;
-  int64_t s3[3];
-  sizes(p, layout, s3);
-  a.n_free = (int)s3[0]; a.n_con = (int)s3[1]; a.nnz = s3[2];
-  colloc_constants(a);
-  D2DX_CUDA(cudaSetDevice(h->device));
-  a.ticket_mode = n_prob < kMaxTickets;        // latency-sensitive single evaluations stay one launch
-  const bool want_cg = (what & (D2DX_EVAL_COST | D2DX_EVAL_GRAD)) != 0;
-  const bool col = want_cg && enabled_h(p->kcol) && n_total > 1;
-  const bool obs = want_cg && enabled_h(p->kobs) && p->n_obs > 0;
-  cudaStream_t st = as_stream(stream);
-  const bool all_pairs_local = col && p->col_all_pairs && pos_all == nullptr;
-  const long per_max = a.nnz > a.n_free ? a.nnz : a.n_free;                    // n_con < n_free
-  const bool idx32 = (long)n_prob * per_max < (1L << 31);
-  if (all_pairs_local && idx32 && pairs_smem_bytes(p->n_ac) <= 200 * 1024) {
-    a.TN = 32; a.APP = kPairWarps; a.ntiles = (p->N + 31) / 32; a.nparts = a.ntiles;
-    const size_t smem = pairs_smem_bytes(p->n_ac);
-    const bool regs = p->n_ac <= 2 * kPairWarps;
-    auto kern = p->n_ac == 2 * kPairWarps ? colloc_pairs_kernel<true, 2 * kPairWarps> : regs ? colloc_pairs_kernel<true> : colloc_pairs_kernel<false>;
-    if (smem > 48 * 1024) D2DX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int warps = p->n_ac < kPairWarps ? p->n_ac : kPairWarps;
-    const dim3 grid = n_prob <= 65535 ? dim3((unsigned)a.ntiles, (unsigned)n_prob) : dim3((unsigned)((long)n_prob * a.ntiles));
-    kern<<<grid, warps * 32, smem, st>>>(a);
-    D2DX_LAUNCH_CHECK("colloc_pairs_kernel");
-  } else {
-    tile_shape(p->n_ac, a.TN, a.APP);
-    a.ntiles = (p->N + a.TN - 1) / a.TN; a.nparts = a.ntiles;
-    const unsigned grid = (unsigned)((long)n_prob * a.ntiles);
-    if (col || obs) {
-      const size_t smem = col ? (size_t)n_total * 2 * a.TN * sizeof(double) : 0;
-      if (smem > 48 * 1024) {
-        D2DX_CHECK_ARG(smem <= 200 * 1024, "%s: %d aircraft need %zu B of shared memory", who, n_total, smem);
-        D2DX_CUDA(cudaFuncSetAttribute(colloc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      }
-      colloc_kernel<true><<<grid, kCollocThreads, smem, st>>>(a);
-    } else {
-      colloc_kernel<false><<<grid, kCollocThreads, 0, st>>>(a);
-    }
-    D2DX_LAUNCH_CHECK("colloc_kernel");
-  }
-  if ((what & D2DX_EVAL_COST) && !a.ticket_mode) {
-    colloc_cost_kernel<<<(n_prob + 3) / 4, 128, 0, st>>>(a, obs, col);
-    D2DX_LAUNCH_CHECK("colloc_cost_kernel");
-  }
-  return D2DX_OK;
-}
-
 }  // namespace d2dx
 
 using namespace d2dx;
@@ -565,18 +492,60 @@ int d2dx_colloc_init_dense(d2dx_handle* h, const d2dx_colloc_problem* p, int32_t
 int d2dx_colloc_eval(d2dx_handle* h, const d2dx_colloc_problem* p, int32_t n_prob, const double* free_, int32_t layout,
                      uint32_t what, double* residual, double* jac, double* cost, double* grad, double* scratch, void* stream) {
   D2DX_NVTX("d2dx_colloc_eval");
-  return launch_eval(h, p, n_prob, p ? p->n_ac : 0, 0, free_, nullptr, layout, what, residual, jac, cost, grad, scratch, stream,
-                     "d2dx_colloc_eval");
-}
-
-int d2dx_colloc_eval_shard(d2dx_handle* h, const d2dx_colloc_problem* p, int32_t n_ac_total, int32_t a_lo,
-                           const double* free_local, const double* pos_all, uint32_t what, double* residual, double* jac,
-                           double* cost, double* grad, double* scratch, void* stream) {
-  D2DX_NVTX("d2dx_colloc_eval_shard");
-  D2DX_CHECK_ARG(p && pos_all && n_ac_total >= p->n_ac && a_lo >= 0 && a_lo + p->n_ac <= n_ac_total,
-                 "d2dx_colloc_eval_shard: shard [%d,+%d) of %d", a_lo, p ? p->n_ac : -1, n_ac_total);
-  return launch_eval(h, p, 1, n_ac_total, a_lo, free_local, pos_all, D2DX_JAC_COMPACT, what, residual, jac, cost, grad, scratch,
-                     stream, "d2dx_colloc_eval_shard");
+  if (int rc = check_problem(p, "d2dx_colloc_eval")) return rc;
+  D2DX_CHECK_ARG(h && free_ && n_prob >= 1 && n_prob <= 65536, "d2dx_colloc_eval: n_prob=%d (1..65536 per call)", n_prob);
+  D2DX_CHECK_ARG(layout == D2DX_JAC_COMPACT || layout == D2DX_JAC_OPTY_DENSE, "d2dx_colloc_eval: unknown Jacobian layout %d", layout);
+  D2DX_CHECK_ARG(!(what & D2DX_EVAL_RESIDUAL) || residual, "d2dx_colloc_eval: residual requested but NULL");
+  D2DX_CHECK_ARG(!(what & D2DX_EVAL_JAC) || jac, "d2dx_colloc_eval: jacobian requested but NULL");
+  D2DX_CHECK_ARG(!(what & D2DX_EVAL_COST) || (cost && scratch), "d2dx_colloc_eval: cost requested but cost/scratch NULL");
+  D2DX_CHECK_ARG(!(what & D2DX_EVAL_GRAD) || grad, "d2dx_colloc_eval: gradient requested but NULL");
+  D2DX_CHECK_ARG(5L * p->n_ac * p->N < (1L << 31), "d2dx_colloc_eval: 5 n_ac N = %ld does not fit 32-bit offsets", 5L * p->n_ac * p->N);
+  CollocArgs a;
+  a.p = *p; a.n_prob = n_prob; a.layout = layout; a.what = what; a.free_ = free_;
+  a.res = residual; a.jac = jac; a.cost = cost; a.grad = grad; a.scratch = scratch;
+  int64_t s3[3];
+  sizes(p, layout, s3);
+  a.n_free = (int)s3[0]; a.n_con = (int)s3[1]; a.nnz = s3[2];
+  colloc_constants(a);
+  D2DX_CUDA(cudaSetDevice(h->device));
+  a.ticket_mode = n_prob < kMaxTickets;        // latency-sensitive single evaluations stay one launch
+  const bool want_cg = (what & (D2DX_EVAL_COST | D2DX_EVAL_GRAD)) != 0;
+  const bool col = want_cg && enabled_h(p->kcol) && p->n_ac > 1;
+  const bool obs = want_cg && enabled_h(p->kobs) && p->n_obs > 0;
+  cudaStream_t st = as_stream(stream);
+  const long per_max = a.nnz > a.n_free ? a.nnz : a.n_free;                    // n_con < n_free
+  const bool idx32 = (long)n_prob * per_max < (1L << 31);
+  if (col && p->col_all_pairs && idx32 && pairs_smem_bytes(p->n_ac) <= 200 * 1024) {
+    a.TN = 32; a.APP = kPairWarps; a.ntiles = (p->N + 31) / 32; a.nparts = a.ntiles;
+    const size_t smem = pairs_smem_bytes(p->n_ac);
+    const bool regs = p->n_ac <= 2 * kPairWarps;
+    auto kern = p->n_ac == 2 * kPairWarps ? colloc_pairs_kernel<true, 2 * kPairWarps> : regs ? colloc_pairs_kernel<true> : colloc_pairs_kernel<false>;
+    if (smem > 48 * 1024) D2DX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int warps = p->n_ac < kPairWarps ? p->n_ac : kPairWarps;
+    const dim3 grid = n_prob <= 65535 ? dim3((unsigned)a.ntiles, (unsigned)n_prob) : dim3((unsigned)((long)n_prob * a.ntiles));
+    kern<<<grid, warps * 32, smem, st>>>(a);
+    D2DX_LAUNCH_CHECK("colloc_pairs_kernel");
+  } else {
+    tile_shape(p->n_ac, a.TN, a.APP);
+    a.ntiles = (p->N + a.TN - 1) / a.TN; a.nparts = a.ntiles;
+    const unsigned grid = (unsigned)((long)n_prob * a.ntiles);
+    if (col || obs) {
+      const size_t smem = col ? (size_t)p->n_ac * 2 * a.TN * sizeof(double) : 0;
+      if (smem > 48 * 1024) {
+        D2DX_CHECK_ARG(smem <= 200 * 1024, "d2dx_colloc_eval: %d aircraft need %zu B of shared memory", p->n_ac, smem);
+        D2DX_CUDA(cudaFuncSetAttribute(colloc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      }
+      colloc_kernel<true><<<grid, kCollocThreads, smem, st>>>(a);
+    } else {
+      colloc_kernel<false><<<grid, kCollocThreads, 0, st>>>(a);
+    }
+    D2DX_LAUNCH_CHECK("colloc_kernel");
+  }
+  if ((what & D2DX_EVAL_COST) && !a.ticket_mode) {
+    colloc_cost_kernel<<<(n_prob + 3) / 4, 128, 0, st>>>(a, obs, col);
+    D2DX_LAUNCH_CHECK("colloc_cost_kernel");
+  }
+  return D2DX_OK;
 }
 
 int d2dx_cost_bank_max(d2dx_handle* h, int32_t n_prob, int32_t n_free, int32_t off_phi, int32_t N, double obj_scale, const double* free_,
@@ -588,16 +557,6 @@ int d2dx_cost_bank_max(d2dx_handle* h, int32_t n_prob, int32_t n_free, int32_t o
   D2DX_CUDA(cudaSetDevice(h->device));
   bank_max_kernel<<<n_prob, 256, 0, as_stream(stream)>>>(n_free, off_phi, N, obj_scale, free_, cost, grad);
   D2DX_LAUNCH_CHECK("bank_max_kernel");
-  return D2DX_OK;
-}
-
-int d2dx_colloc_pack_positions(d2dx_handle* h, int32_t n_ac, int32_t N, const double* free_local, double* pos, void* stream) {
-  D2DX_NVTX("d2dx_colloc_pack_positions");
-  D2DX_CHECK_ARG(h && n_ac >= 1 && N >= 1 && free_local && pos, "d2dx_colloc_pack_positions: bad argument");
-  D2DX_CUDA(cudaSetDevice(h->device));
-  const long total = (long)n_ac * 2 * N;
-  pack_positions_kernel<<<(int)((total + 255) / 256 < 2048 ? (total + 255) / 256 : 2048), 256, 0, as_stream(stream)>>>(n_ac, N, free_local, pos);
-  D2DX_LAUNCH_CHECK("pack_positions_kernel");
   return D2DX_OK;
 }
 

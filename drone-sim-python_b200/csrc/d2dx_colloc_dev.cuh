@@ -12,8 +12,6 @@ struct CollocArgs {
   uint32_t what;
   const double* free_;
   double *res, *jac, *cost, *grad, *scratch;   // scratch: [kTicketDoubles of int32 tickets][per-block cost partials]
-  int n_total, a_lo;          // shard context: owned aircraft are global [a_lo, a_lo + p.n_ac) of n_total
-  const double* pos_all;      // [n_total][2][N] or NULL (positions come from free_)
   int TN, APP, ntiles;        // nodes per tile, aircraft per pass, tiles per problem
   int ticket_mode;            // 1: the last block of a problem (atomic ticket) finishes the cost in this kernel;
                               // 0: per-block partials only, colloc_cost_kernel finishes (large batches: no fence in the hot kernel)

@@ -16,7 +16,7 @@
 // 8-byte words {half of the bits, evaluation number}; an 8-byte store arrives whole, so a receiver that reads both
 // evaluation numbers it expects holds valid data -- no memory fence (MEMBAR.SYS cost ~4 us per use in the fence + flag
 // version, profiles/r2_sharded_c4.md), no separate flag, one NVLink traversal of latency.  Twice the bytes, of a 128 kB
-// exchange.  There is no collective call, no pack kernel and no host synchronisation; the evaluation number lives on the
+// exchange.  There is no collective call and no host synchronisation; the evaluation number lives on the
 // device, so the launch can be captured in a CUDA graph and replayed.  Phase 4 doubles as the barrier that keeps
 // evaluation e + 1 from overwriting tables a slower rank still reads in evaluation e.
 // A peer that never answers costs `spin_cycles` per wait and is reported by d2dx_peer_status (never a hang).
@@ -47,7 +47,8 @@ struct PeerCtrl {
 };
 
 struct PeerArgs {
-  CollocArgs c;                  // c.p = the local shard as a problem of n_own aircraft; c.n_total, c.a_lo; outputs shard-local
+  CollocArgs c;                  // c.p = the local shard as a problem of n_own aircraft; outputs shard-local
+  int n_total, a_lo;             // owned aircraft are global [a_lo, a_lo + c.p.n_ac) of n_total
   int world, rank, max_prob, ntiles;
   unsigned char* base[D2DX_PEER_MAX_WORLD];
   size_t off_cpart, off_lpart, off_pos;
@@ -88,7 +89,7 @@ __global__ void __launch_bounds__(kPeerWarps * 32, 3) colloc_peer_kernel(const _
   extern __shared__ double sm[];                   // [n_total][2][32] positions, then [W][4] reduction scratch
   const CollocArgs& a = g.c;
   const d2dx_colloc_problem& P = a.p;
-  const int N = P.N, n_own = P.n_ac, n_total = a.n_total;
+  const int N = P.N, n_own = P.n_ac, n_total = g.n_total;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, W = blockDim.x >> 5;
   double* spos = sm + lane;
   double* sred = sm + n_total * 64;
@@ -115,7 +116,7 @@ __global__ void __launch_bounds__(kPeerWarps * 32, 3) colloc_peer_kernel(const _
         const double* fr = a.free_ + (size_t)prob * a.n_free;
         for (int a_l = w; a_l < n_own; a_l += W) {
           const double x = fr[(3 * a_l) * N + i], y = fr[(3 * a_l + 1) * N + i];
-          const size_t o = ((((size_t)prob * n_total + a.a_lo + a_l) * 2) * N + i) * 2;      // two words per value
+          const size_t o = ((((size_t)prob * n_total + g.a_lo + a_l) * 2) * N + i) * 2;      // two words per value
           for (int r = 0; r < g.world; ++r) {
             if (r == g.rank) continue;
             unsigned long long* dst = reinterpret_cast<unsigned long long*>(g.base[r] + g.off_pos);
@@ -137,7 +138,7 @@ __global__ void __launch_bounds__(kPeerWarps * 32, 3) colloc_peer_kernel(const _
 
     if (use_col) {                                 // the owned positions of this tile into shared memory
       for (int a_l = w; a_l < n_own; a_l += W) {
-        const int gl = a.a_lo + a_l;
+        const int gl = g.a_lo + a_l;
         double x = 0.0, y = 0.0;
         if (valid) { x = fr[(3 * a_l) * N + i]; y = fr[(3 * a_l + 1) * N + i]; }
         spos[(gl * 2) * 32] = x; spos[(gl * 2 + 1) * 32] = y;
@@ -158,7 +159,7 @@ __global__ void __launch_bounds__(kPeerWarps * 32, 3) colloc_peer_kernel(const _
     if (use_col) {
       bool arrived = true;
       for (int gl = w; gl < n_total; gl += W) {
-        if (gl >= a.a_lo && gl < a.a_lo + n_own) continue;
+        if (gl >= g.a_lo && gl < g.a_lo + n_own) continue;
         double x = 0.0, y = 0.0;
         if (valid) {
           const size_t o = ((((size_t)prob * n_total + gl) * 2) * N + i) * 2;
@@ -175,7 +176,7 @@ __global__ void __launch_bounds__(kPeerWarps * 32, 3) colloc_peer_kernel(const _
     // ---- phase 3: obstacle and collision terms of the owned aircraft, gradient of x, y ----
     if (want_cg && valid) {
       for (int a_l = w; a_l < n_own; a_l += W) {
-        const int gl = a.a_lo + a_l;
+        const int gl = g.a_lo + a_l;
         const int ox = 3 * a_l * N + i;
         const double x = fr[ox], y = fr[ox + N];
         double gx = 0.0, gy = 0.0;
@@ -406,10 +407,10 @@ int d2dx_colloc_eval_peer(d2dx_handle* h, d2dx_peer* peer, const d2dx_colloc_pro
   CollocArgs& a = g.c;
   a.p = *p; a.n_prob = n_prob; a.layout = D2DX_JAC_COMPACT; a.what = what; a.free_ = free_local;
   a.res = residual; a.jac = jac; a.cost = cost; a.grad = grad; a.scratch = nullptr;
-  a.n_total = peer->n_total; a.a_lo = a_lo; a.pos_all = nullptr;
   a.TN = 32; a.APP = kPeerWarps; a.ntiles = peer->ntiles; a.nparts = peer->ntiles; a.ticket_mode = 1;
   a.n_free = 5 * p->n_ac * p->N; a.n_con = 3 * p->n_ac * (p->N - 1) + p->n_inst; a.nnz = 12L * p->n_ac * (p->N - 1) + p->n_inst;
   colloc_constants(a);
+  g.n_total = peer->n_total; g.a_lo = a_lo;
   g.world = peer->world; g.rank = peer->rank; g.max_prob = peer->max_prob; g.ntiles = peer->ntiles;
   for (int r = 0; r < peer->world; ++r) g.base[r] = peer->base[r];
   g.off_cpart = peer->off_cpart; g.off_lpart = peer->off_lpart; g.off_pos = peer->off_pos;

@@ -141,8 +141,6 @@ def _load():
         "d2dx_colloc_scratch_size": (i64, [P(CollocProblem), i32]),
         "d2dx_colloc_eval": (C.c_int, [H, P(CollocProblem), i32, c_dp, i32, u32, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
         "d2dx_cost_bank_max": (C.c_int, [H, i32, i32, i32, i32, dbl, c_dp, c_dp, c_dp, c_dp]),
-        "d2dx_colloc_eval_shard": (C.c_int, [H, P(CollocProblem), i32, i32, c_dp, c_dp, u32, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
-        "d2dx_colloc_pack_positions": (C.c_int, [H, i32, i32, c_dp, c_dp, c_dp]),
         "d2dx_peer_create": (C.c_int, [H, i32, i32, i32, i32, i32, P(H)]),
         "d2dx_peer_ipc_handle": (C.c_int, [H, C.c_char_p]),
         "d2dx_peer_connect_ipc": (C.c_int, [H, C.c_char_p]),

@@ -5,10 +5,7 @@
 * One multi-aircraft collocation problem shards by aircraft: the only exchange is the aircraft positions
   (n_ac*N*2 doubles) before the pairwise collision terms and the four cost sums; residual / Jacobian / gradient
   rows stay with the rank that owns the aircraft.  The exchange is done by the evaluation kernel itself through
-  NVLink peer memory (backend "peer"), or by an all-gather + all-reduce around the shard kernel ("collective").
-
-The compute backend is the engine (CUDA); the class takes it as an argument so the host-side sharding logic can
-be exercised on CPU under gloo with a stand-in (tests/test_distributed_cpu.py)."""
+  NVLink peer memory, so the GPUs of the job must have peer access to each other (one NVLink box)."""
 import numpy as np
 import torch
 import torch.distributed as dist
@@ -57,13 +54,15 @@ class ShardedCollocation:
     """Aircraft-sharded evaluation of ONE problem (or a batch of `max_prob` problems) across the ranks of `group`.
     Every rank must own the same number of aircraft.
 
-    backend "peer" (default on the CUDA engine): ONE kernel per evaluation and rank -- positions and cost partials travel
-    as peer-memory stores over NVLink with per-tile flags (d2dx_colloc_eval_peer, include/d2dx.h); `graph()` captures it
-    in a CUDA graph.  backend "collective": pack kernel + all_gather_into_tensor + shard kernel + all_reduce (the
-    torch.distributed formulation; also what the CPU/gloo host-logic test drives through a stand-in engine)."""
+    ONE kernel per evaluation and rank: positions and cost partials travel as peer-memory stores over NVLink, each value
+    tagged with the evaluation number (d2dx_colloc_eval_peer, include/d2dx.h); `graph()` captures it in a CUDA graph.
+    connect=True maps every rank's exchange buffer through CUDA IPC over torch.distributed; with connect=False the
+    caller connects the exchange objects itself (`emulate_peer_eval`: every rank in one process)."""
 
     def __init__(self, n_ac, N, h, wind, inst, cost, obj_scale=1., engine=None, group=None, world=None, rank=None,
-                 problem_factory=None, backend=None, max_prob=1, peers=None):
+                 max_prob=1, connect=True):
+        from .collocation import CollocationProblem
+        from .engine import get_engine
         self.group = group
         self.world = world if world is not None else (dist.get_world_size(group) if dist.is_initialized() else 1)
         self.rank = rank if rank is not None else (dist.get_rank(group) if dist.is_initialized() else 0)
@@ -71,65 +70,35 @@ class ShardedCollocation:
             raise ValueError(f"{n_ac} aircraft do not split evenly over {self.world} ranks")
         self.n_ac, self.N, self.max_prob = n_ac, N, int(max_prob)
         self.shard = AircraftShard(n_ac, N, list(inst), self.world, self.rank)
-        if backend is None:
-            backend = "collective" if problem_factory is not None else "peer"
-        self.backend = backend
-        if problem_factory is None:
-            from .collocation import CollocationProblem
-            from .engine import get_engine
-            engine = engine or get_engine()
-            problem_factory = CollocationProblem
-        self.eng = engine
+        self.eng = e = engine or get_engine()
         cost.in_div = n_ac                                   # CostInput normalises by the TOTAL aircraft count
-        self.local = problem_factory(self.shard.n_own, N, h, wind=wind, inst=self.shard.inst_local, cost=cost,
-                                     obj_scale=obj_scale, layout="compact", multi=True, engine=engine)
-        e, P = self.eng, self.max_prob
+        self.local = CollocationProblem(self.shard.n_own, N, h, wind=wind, inst=self.shard.inst_local, cost=cost,
+                                        obj_scale=obj_scale, layout="compact", multi=True, engine=e)
+        P = self.max_prob
         self.res = e.empty(P, self.local.num_constraints); self.jac = e.empty(P, self.local.nnz)
         self.grad = e.empty(P, self.local.num_free); self.cost = e.zeros(P)
-        if backend == "peer":
-            self.peer = e.peer_create(self.world, self.rank, P, n_ac, N)
-            if peers is not None:                            # single-process emulation: the caller connects the objects
-                pass
-            elif self.world > 1:
-                handles = [None] * self.world
-                dist.all_gather_object(handles, self.peer.ipc_handle(), group=group)
-                self.peer.connect_ipc(handles)
-                dist.barrier(group=group)                    # nobody launches before every rank has mapped every buffer
-        else:
-            if P != 1:
-                raise ValueError("the collective backend evaluates one problem per call")
-            self.pos_local = e.empty(self.shard.n_own, 2, N)
-            self.pos_all = e.empty(n_ac, 2, N)
-            self.scratch = e.colloc_scratch(self.local.c, 1)
+        self.peer = e.peer_create(self.world, self.rank, P, n_ac, N)
+        if connect and self.world > 1:
+            handles = [None] * self.world
+            dist.all_gather_object(handles, self.peer.ipc_handle(), group=group)
+            self.peer.connect_ipc(handles)
+            dist.barrier(group=group)                        # nobody launches before every rank has mapped every buffer
 
     def evaluate(self, free_local, what=_lib.EVAL_ALL):
         """free_local: this rank's slice (device tensor, shard-local planner layout), (num_free_local,) or
         (n_prob, num_free_local).  Returns (residual_local, jac_local, cost_total, grad_local) as device tensors (leading
         problem axis only for 2-D input)."""
-        e = self.eng
-        if self.backend == "peer":
-            single = free_local.dim() == 1
-            n_prob = 1 if single else free_local.shape[0]
-            e.colloc_eval_peer(self.peer, self.local.c, n_prob, self.shard.a_lo, free_local, what, self.res, self.jac, self.cost, self.grad)
-            if single:
-                return self.res[0], self.jac[0], self.cost[:1], self.grad[0]
-            return self.res[:n_prob], self.jac[:n_prob], self.cost[:n_prob], self.grad[:n_prob]
-        e.colloc_pack_positions(self.shard.n_own, self.N, free_local, self.pos_local)
-        if self.world > 1:
-            dist.all_gather_into_tensor(self.pos_all, self.pos_local, group=self.group)      # the one exchange step
-        else:
-            self.pos_all.copy_(self.pos_local)
-        e.colloc_eval_shard(self.local.c, self.n_ac, self.shard.a_lo, free_local, self.pos_all, what,
-                            self.res[0], self.jac[0], self.cost, self.grad[0], self.scratch)
-        if self.world > 1 and (what & _lib.EVAL_COST):
-            dist.all_reduce(self.cost, op=dist.ReduceOp.SUM, group=self.group)
-        return self.res[0], self.jac[0], self.cost, self.grad[0]
+        single = free_local.dim() == 1
+        n_prob = 1 if single else free_local.shape[0]
+        self.eng.colloc_eval_peer(self.peer, self.local.c, n_prob, self.shard.a_lo, free_local, what, self.res, self.jac, self.cost,
+                                  self.grad)
+        if single:
+            return self.res[0], self.jac[0], self.cost[:1], self.grad[0]
+        return self.res[:n_prob], self.jac[:n_prob], self.cost[:n_prob], self.grad[:n_prob]
 
     def graph(self, free_local, what=_lib.EVAL_ALL):
-        """Captures one evaluation (peer backend) in a CUDA graph: returns (replay, outputs).  Every rank must replay the
-        same number of times."""
-        if self.backend != "peer":
-            raise ValueError("graph capture needs the peer backend (collectives are not captured here)")
+        """Captures one evaluation in a CUDA graph: returns (replay, outputs).  Every rank must replay the same number of
+        times."""
         out = self.evaluate(free_local, what)                 # warm-up outside the capture (every rank: one evaluation)
         torch.cuda.synchronize(self.eng.device)
         g = torch.cuda.CUDAGraph()
@@ -140,12 +109,10 @@ class ShardedCollocation:
 
     def check(self):
         """Raises if a peer ever failed to answer (the kernel gives up after ~1 s per wait instead of hanging)."""
-        if self.backend == "peer":
-            st = self.peer.status()
-            if st["timeouts"]:
-                raise RuntimeError(f"rank {self.rank}: {st['timeouts']} peer waits timed out; outputs are invalid")
-            return st
-        return {}
+        st = self.peer.status()
+        if st["timeouts"]:
+            raise RuntimeError(f"rank {self.rank}: {st['timeouts']} peer waits timed out; outputs are invalid")
+        return st
 
 
 def emulate_peer_eval(n_ac, N, h, wind, inst, cost, free, world, engine=None, replays=2):
@@ -158,8 +125,8 @@ def emulate_peer_eval(n_ac, N, h, wind, inst, cost, free, world, engine=None, re
     inst = list(inst)
     free = np.asarray(free, dtype=np.float64).reshape(-1, 5 * n_ac * N)
     P = len(free)
-    scs = [ShardedCollocation(n_ac, N, h, wind, inst, copy.copy(cost), engine=eng, world=world, rank=r, backend="peer", max_prob=P,
-                              peers=True) for r in range(world)]
+    scs = [ShardedCollocation(n_ac, N, h, wind, inst, copy.copy(cost), engine=eng, world=world, rank=r, max_prob=P, connect=False)
+           for r in range(world)]
     for sc in scs:
         sc.peer.connect_local([q.peer for q in scs])
     fls = [eng.to_device(np.ascontiguousarray(free[:, sc.shard.idx_free])) for sc in scs]
@@ -178,31 +145,4 @@ def emulate_peer_eval(n_ac, N, h, wind, inst, cost, free, world, engine=None, re
         out["grad"][:, sc.shard.idx_free] = sc.grad.cpu().numpy()
         out["cost"].append(sc.cost.cpu().numpy().copy())
         out["status"].append(sc.peer.status())
-    return out
-
-
-def emulate_sharded_eval(n_ac, N, h, wind, inst, cost, free, world, engine=None):
-    """Runs every rank's shard kernel in turn on ONE GPU (positions "gathered" by slicing the global free vector)
-    and reassembles the global vectors.  Used to check the shard kernel without `world` GPUs."""
-    from .collocation import CollocationProblem
-    from .engine import get_engine
-    import copy
-    eng = engine or get_engine()
-    inst = list(inst)
-    free = np.asarray(free, dtype=np.float64)
-    n_con, nnz = 3 * n_ac * (N - 1) + len(inst), 12 * n_ac * (N - 1) + len(inst)
-    out = {"residual": np.zeros(n_con), "jac": np.zeros(nnz), "grad": np.zeros(free.size), "cost": 0.}
-    pos_all = eng.empty(n_ac, 2, N)
-    eng.colloc_pack_positions(n_ac, N, eng.to_device(free), pos_all)
-    for rank in range(world):
-        sh = AircraftShard(n_ac, N, inst, world, rank)
-        c = copy.copy(cost); c.in_div = n_ac
-        loc = CollocationProblem(sh.n_own, N, h, wind=wind, inst=sh.inst_local, cost=c, layout="compact", multi=True, engine=eng)
-        fl = eng.to_device(free[sh.idx_free])
-        res, jac, grad, cst = eng.empty(loc.num_constraints), eng.empty(loc.nnz), eng.empty(loc.num_free), eng.zeros(1)
-        eng.colloc_eval_shard(loc.c, n_ac, sh.a_lo, fl, pos_all, _lib.EVAL_ALL, res, jac, cst, grad, eng.colloc_scratch(loc.c, 1))
-        out["residual"][sh.idx_con] = res.cpu().numpy()
-        out["jac"][sh.idx_jac] = jac.cpu().numpy()
-        out["grad"][sh.idx_free] = grad.cpu().numpy()
-        out["cost"] += float(cst.cpu().numpy()[0])
     return out

@@ -282,16 +282,6 @@ class Engine:
         self.launches += 1
         return cost, grad
 
-    def colloc_eval_shard(self, prob_local, n_ac_total, a_lo, free_local, pos_all, what, residual, jac, cost, grad, scratch):
-        check(lib.d2dx_colloc_eval_shard(self.h, C.byref(prob_local), n_ac_total, a_lo, _ptr(free_local), _ptr(pos_all), what,
-                                         _ptr(residual), _ptr(jac), _ptr(cost), _ptr(grad), _ptr(scratch), self.stream_ptr()),
-              "d2dx_colloc_eval_shard")
-        self.launches += 1
-
-    def colloc_pack_positions(self, n_ac, N, free_local, pos):
-        check(lib.d2dx_colloc_pack_positions(self.h, n_ac, N, _ptr(free_local), _ptr(pos), self.stream_ptr()), "d2dx_colloc_pack_positions")
-        self.launches += 1
-
 
     # ---- peer exchange (aircraft-sharded collocation over NVLink peer memory) -------------------------------
     def peer_create(self, world, rank, max_prob, n_ac_total, N):

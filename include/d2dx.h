@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define D2DX_VERSION 102
+#define D2DX_VERSION 103
 
 enum { D2DX_OK = 0, D2DX_EINVAL = 1, D2DX_ECUDA = 2, D2DX_EUNSUPPORTED = 3 };
 
@@ -309,29 +309,14 @@ int d2dx_colloc_eval(d2dx_handle* h, const d2dx_colloc_problem* p_host, int32_t 
  * cost or grad may be NULL. */
 int d2dx_cost_bank_max(d2dx_handle* h, int32_t n_prob, int32_t n_free, int32_t off_phi, int32_t N, double obj_scale,
                        const double* free_, double* cost, double* grad, void* stream);
-/* Aircraft-sharded evaluation of ONE problem (SURVEY 8e).  `p_local_host` describes THIS rank's shard as a
- * problem of n_ac = number of owned aircraft (free_local, residual, jac (compact layout), grad all use the
- * shard-local layout; in_div must be the TOTAL aircraft count).  The owned aircraft are global aircraft
- * [a_lo, a_lo + n_ac) of n_ac_total; pos_all[n_ac_total][2][N] holds every aircraft's x,y -- the
- * all-gathered positions, each rank contributing its contiguous [n_own][2][N] chunk.  cost[0] receives this
- * rank's share (own input terms, obstacles if it owns aircraft 0, each pair counted once at the owner of
- * its lower-index aircraft); the caller all-reduces it. */
-int d2dx_colloc_eval_shard(d2dx_handle* h, const d2dx_colloc_problem* p_local_host, int32_t n_ac_total,
-                           int32_t a_lo, const double* free_local, const double* pos_all, uint32_t what,
-                           double* residual, double* jac, double* cost, double* grad, double* scratch,
-                           void* stream);
-/* packs the x,y slices of a (shard-local) free vector into pos[n_ac][2][N], the all-gather send buffer */
-int d2dx_colloc_pack_positions(d2dx_handle* h, int32_t n_ac, int32_t N, const double* free_local,
-                               double* pos, void* stream);
-
 /* -------- aircraft-sharded evaluation over NVLink peer memory: ONE kernel per rank, no collective call (SURVEY 8e) --------
  * The exchange step the north star names ("all-gather aircraft positions for the cross-shard avoidance terms, reduce
  * costs") done by the evaluation kernel itself: each rank stores its aircraft's x, y straight from free_local into every
  * peer's position table (peer memory), computes everything local while the stores travel, reads the peers' tiles from its
  * own table (every value travels with the evaluation number in the same 8-byte words, so arrival needs neither a fence nor
  * a flag), adds the collision terms, and the block of a problem's last tile exchanges the four cost sums the same way, so
- * that every rank ends with the identical total cost[n_prob].  Replaces d2dx_colloc_pack_positions + all-gather + d2dx_colloc_eval_shard
- * + all-reduce for the callbacks of 07_multioptyplan.py:69-78 when one problem is spread over the GPUs of a box.
+ * that every rank ends with the identical total cost[n_prob].  Serves the callbacks of 07_multioptyplan.py:69-78 when one
+ * problem is spread over the GPUs of a box.
  *
  * d2dx_peer_create allocates this rank's exchange buffer (the only allocation; capacity: max_prob problems of n_ac_total
  * aircraft x N nodes).  Between processes the ranks swap d2dx_peer_ipc_handle blobs (64 bytes each, e.g. with
@@ -354,8 +339,10 @@ int d2dx_peer_status(d2dx_peer* p, int32_t* status_host4);
  * 6 every rank's sums arrived, 7 block 0 leaves -- where the latency of a sharded evaluation goes */
 int d2dx_peer_timeline(d2dx_peer* p, uint64_t* stamps_host8);
 int d2dx_peer_destroy(d2dx_peer* p);
-/* p_local_host / free_local / residual / jac (compact) / grad as in d2dx_colloc_eval_shard, for n_prob problems stacked on
- * a leading axis; cost[n_prob] receives the TOTAL cost of each problem (all ranks' shares, summed in rank order). */
+/* `p_local_host` describes THIS rank's shard as a problem of n_ac = number of owned aircraft (in_div must be the TOTAL
+ * aircraft count); the owned aircraft are global aircraft [a_lo, a_lo + n_ac) of the exchange's n_ac_total.  free_local,
+ * residual, jac (compact layout) and grad use the shard-local layout, for n_prob problems stacked on a leading axis;
+ * cost[n_prob] receives the TOTAL cost of each problem (all ranks' shares, summed in rank order). */
 int d2dx_colloc_eval_peer(d2dx_handle* h, d2dx_peer* peer, const d2dx_colloc_problem* p_local_host, int32_t n_prob,
                           int32_t a_lo, const double* free_local, uint32_t what, double* residual, double* jac,
                           double* cost, double* grad, void* stream);

@@ -1,73 +1,36 @@
-"""world_size-2 gloo test of the aircraft-sharded collocation driver (host-side logic: index maps, the
-all-gather of positions, the all-reduce of the cost).  The CUDA engine is replaced by a stand-in that computes
-the shard quantities with the oracle -- test infrastructure only."""
+"""Host-side logic of the multi-GPU plumbing without a GPU: the index maps of an aircraft shard against the oracle, and a
+world_size-2 gloo run of the population-statistics reduction and the unit partition."""
 import os
 import socket
 
 import numpy as np
-import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from oracle import d2d_oracle as orc
 
-N_AC, N, H = 4, 12, 0.1
-SPEC = dict(vsp=12., kvel=3., kbank=2., kcol=10., rcol=10., pairs="all", kobs=1.5, obstacles=[(1., 2., 6.)], obs_kind=1)
+N_AC, N, H, WIND = 4, 12, 0.1, (0.5, -1.)
 
 
-class _Dummy:
-    pass
-
-
-class OracleEngine:
-    """Implements the handful of engine methods ShardedCollocation uses, on CPU tensors."""
-
-    def empty(self, *shape, dtype=torch.float64): return torch.zeros(*shape, dtype=dtype)
-    def zeros(self, *shape, dtype=torch.float64): return torch.zeros(*shape, dtype=dtype)
-    def colloc_scratch(self, prob, n): return torch.zeros(1, dtype=torch.float64)
-
-    def colloc_pack_positions(self, n_ac, n, free_local, pos):
-        f = free_local.numpy()
-        pos.copy_(torch.from_numpy(np.stack([np.stack([f[(3 * a) * n:(3 * a + 1) * n], f[(3 * a + 1) * n:(3 * a + 2) * n]]) for a in range(n_ac)])))
-
-    def colloc_eval_shard(self, prob, n_total, a_lo, free_local, pos_all, what, res, jac, cost, grad, scratch):
-        n_own, f, P = prob.n_ac, free_local.numpy(), pos_all.numpy()
-        res.copy_(torch.from_numpy(orc.colloc_residual(f, N, n_own, H, (0.5, -1.), prob.inst)))
-        jac.copy_(torch.from_numpy(np.concatenate([orc.colloc_jac_compact(f, N, n_own, H).reshape(-1), np.ones(len(prob.inst))])))
-        # global free vector: every aircraft's x, y from the gathered positions, own psi/phi/v, zeros elsewhere
-        sx, sy, sp, sphi, sv = orc.multi_slices(N, n_total)
-        lx, ly, lp, lphi, lv = orc.multi_slices(N, n_own)
-        G = np.zeros(5 * n_total * N)
-        for g_ in range(n_total):
-            G[sx[g_]], G[sy[g_]] = P[g_, 0], P[g_, 1]
-        own = range(a_lo, a_lo + n_own)
-        for k, g_ in enumerate(own):
-            G[sp[g_]], G[sphi[g_]], G[sv[g_]] = f[lp[k]], f[lphi[k]], f[lv[k]]
-        c_full, g_full = orc.cost_and_grad(G, N, n_total, SPEC, multi=True)
-        # this rank's share of the cost: own input terms + obstacles if it owns aircraft 0 + pairs whose lower index it owns
-        share = 0.
-        for g_ in own:
-            share += (3. * np.sum(np.square(G[sv[g_]] - 12.)) + 2. * np.sum(np.square(G[sphi[g_]]))) / N / n_total
-            for b in range(g_ + 1, n_total):
-                dx, dy = G[sx[g_]] - G[sx[b]], G[sy[g_]] - G[sy[b]]
-                share += 10. / N * np.sum(np.exp(-(np.square(dx / 10. * 2.) + np.square(dy / 10. * 2.))))
-        if a_lo == 0:
-            dx, dy = G[sx[0]] - 1., G[sy[0]] - 2.
-            share += 1.5 / N * np.sum(np.exp(-(np.square(dx / 6. * 2.) + np.square(dy / 6. * 2.))))
-        # subtract the other aircraft's input terms that G's zeros produced? they are not in `share` by construction
-        cost[0] = share
-        gl = np.zeros(5 * n_own * N)
-        for k, g_ in enumerate(own):
-            gl[lx[k]], gl[ly[k]], gl[lp[k]], gl[lphi[k]], gl[lv[k]] = g_full[sx[g_]], g_full[sy[g_]], g_full[sp[g_]], g_full[sphi[g_]], g_full[sv[g_]]
-        grad.copy_(torch.from_numpy(gl))
-
-
-def fake_problem(n_ac, n, h, wind, inst, cost, obj_scale, layout, multi, engine):
-    p = _Dummy()
-    p.c = _Dummy(); p.c.n_ac = n_ac; p.c.inst = list(inst)
-    p.num_free, p.num_constraints, p.nnz = 5 * n_ac * n, 3 * n_ac * (n - 1) + len(inst), 12 * n_ac * (n - 1) + len(inst)
-    return p
+def test_aircraft_shard_index_maps_against_oracle():
+    """Every rank's shard-local problem (free[idx_free], inst_local), evaluated by the oracle and scattered through idx_con /
+    idx_jac, reproduces the residual and compact Jacobian of the whole problem."""
+    from d2d_b200.distributed import AircraftShard
+    rng = np.random.default_rng(4)
+    free = rng.normal(0, 6., 5 * N_AC * N); free[4 * N_AC * N:] += 12.
+    inst = [(3 * a + k, 0, 1. + a) for a in range(N_AC) for k in range(3)] + [(3 * a + k, N - 1, -1. - a) for a in range(N_AC) for k in range(3)]
+    world = 2
+    res_o = orc.colloc_residual(free, N, N_AC, H, WIND, inst)
+    jac_o = np.concatenate([orc.colloc_jac_compact(free, N, N_AC, H).reshape(-1), np.ones(len(inst))])
+    res, jac = np.full_like(res_o, np.nan), np.full_like(jac_o, np.nan)
+    for r in range(world):
+        sh = AircraftShard(N_AC, N, inst, world, r)
+        fl = free[sh.idx_free]
+        res[sh.idx_con] = orc.colloc_residual(fl, N, sh.n_own, H, WIND, sh.inst_local)
+        jac[sh.idx_jac] = np.concatenate([orc.colloc_jac_compact(fl, N, sh.n_own, H).reshape(-1), np.ones(len(sh.inst_local))])
+    np.testing.assert_allclose(res, res_o, rtol=1e-13, atol=1e-13)
+    np.testing.assert_allclose(jac, jac_o, rtol=1e-13)
 
 
 def _free_port():
@@ -75,39 +38,20 @@ def _free_port():
     return port
 
 
-def _worker(rank, world, port, free, inst, ret):
+def _worker(rank, world, port, ret):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    from d2d_b200.collocation_spec import CostSpec
-    from d2d_b200.distributed import ShardedCollocation, reduce_population_stats, shard_range
-    sc = ShardedCollocation(N_AC, N, H, (0.5, -1.), inst, CostSpec(), engine=OracleEngine(), problem_factory=fake_problem)
-    fl = torch.from_numpy(free[sc.shard.idx_free].copy())
-    res, jac, cost, grad = sc.evaluate(fl)
+    from d2d_b200.distributed import reduce_population_stats, shard_range
     pop = torch.tensor([float(rank + 1), float(10 * (rank + 1))], dtype=torch.float64)
     reduce_population_stats(pop)
-    ret[rank] = dict(res=res.numpy().copy(), jac=jac.numpy().copy(), cost=float(cost[0]), grad=grad.numpy().copy(),
-                     idx_free=sc.shard.idx_free, idx_con=sc.shard.idx_con, idx_jac=sc.shard.idx_jac, pop=pop.numpy().copy(),
-                     rng=shard_range(10, world, rank))
+    ret[rank] = dict(pop=pop.numpy().copy(), rng=shard_range(10, world, rank))
     dist.destroy_process_group()
 
 
-def test_sharded_collocation_two_ranks_gloo():
-    rng = np.random.default_rng(4)
-    free = rng.normal(0, 6., 5 * N_AC * N); free[4 * N_AC * N:] += 12.
-    inst = [(3 * a + k, 0, 1. + a) for a in range(N_AC) for k in range(3)] + [(3 * a + k, N - 1, -1. - a) for a in range(N_AC) for k in range(3)]
+def test_population_stats_two_ranks_gloo():
     world = 2
     mgr = mp.Manager(); ret = mgr.dict()
-    mp.spawn(_worker, args=(world, _free_port(), free, inst, ret), nprocs=world, join=True)
-    res_o = orc.colloc_residual(free, N, N_AC, H, (0.5, -1.), inst)
-    jac_o = np.concatenate([orc.colloc_jac_compact(free, N, N_AC, H).reshape(-1), np.ones(len(inst))])
-    c_o, g_o = orc.cost_and_grad(free, N, N_AC, SPEC, multi=True)
-    res, jac, grad = np.full_like(res_o, np.nan), np.full_like(jac_o, np.nan), np.full_like(g_o, np.nan)
+    mp.spawn(_worker, args=(world, _free_port(), ret), nprocs=world, join=True)
     for r in range(world):
-        o = ret[r]
-        res[o["idx_con"]] = o["res"]; jac[o["idx_jac"]] = o["jac"]; grad[o["idx_free"]] = o["grad"]
-        np.testing.assert_allclose(o["cost"], c_o, rtol=1e-12)          # all-reduced: every rank holds the total
-        np.testing.assert_array_equal(o["pop"], [3., 20.])              # sum / max over ranks
-    np.testing.assert_allclose(res, res_o, rtol=1e-13, atol=1e-13)
-    np.testing.assert_allclose(jac, jac_o, rtol=1e-13)
-    np.testing.assert_allclose(grad, g_o, rtol=1e-12, atol=1e-14)
+        np.testing.assert_array_equal(ret[r]["pop"], [3., 20.])          # sum / max over ranks, on every rank
     assert ret[0]["rng"] == (0, 5) and ret[1]["rng"] == (5, 10)

@@ -167,24 +167,6 @@ def test_opty_name_sorted_input_order(golden):
     assert jd.shape[1] == (N - 1) * 3 * n_ac * 8 * n_ac and np.count_nonzero(jd[0]) <= 12 * n_ac * (N - 1)
 
 
-def test_sharded_evaluation_single_gpu_emulation(golden):
-    """The aircraft-sharded entry point (C4 over 8 ranks, 2 aircraft each) emulated on one GPU: per-shard
-    outputs concatenated = the unsharded evaluation; shard costs sum to the total."""
-    from d2d_b200.collocation import CollocationProblem, CostSpec
-    from d2d_b200 import distributed
-    g = golden["colloc"]
-    n_ac, N, h = 16, 500, 0.02
-    free, inst = g["c4/free"], _inst(g, "c4")
-    cs = CostSpec(vsp=12., kvel=70., kbank=1., kcol=10., rcol=10., all_pairs=True, kobs=0.5, obstacles=[(60., 5., 12.)], obs_kind=1)
-    full = CollocationProblem(n_ac, N, h, inst=inst, cost=cs)
-    res, jac, cost, grad = full.evaluate(free)
-    parts = distributed.emulate_sharded_eval(n_ac, N, h, (0., 0.), inst, cs, free, world=8)
-    np.testing.assert_allclose(parts["residual"], res, rtol=0, atol=0)
-    np.testing.assert_allclose(parts["jac"], jac, rtol=0, atol=0)
-    np.testing.assert_allclose(parts["grad"], grad, rtol=1e-14, atol=1e-16)
-    np.testing.assert_allclose(parts["cost"], cost, rtol=1e-13)
-
-
 def test_planner_front_ends_and_cost_classes(golden):
     """The mirrored Planner / cost classes used the way the reference scripts use them (06_optyplan.py:177-204,
     test/test_objective.py): known-answer costs of SURVEY appendix C, instance constraints, triangle guess."""

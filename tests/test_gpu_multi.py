@@ -1,5 +1,6 @@
 """Two-GPU tests (skipped on a single-GPU box): the aircraft-sharded collocation evaluation (fused peer-memory kernel over
-NVLink, its CUDA-graph replay, and the NCCL all-gather + all-reduce formulation), and scenario-sharded rollouts with the final statistics reduction."""
+NVLink and its CUDA-graph replay, against the unsharded evaluation), and scenario-sharded rollouts with the final statistics
+reduction."""
 import os
 import socket
 
@@ -37,11 +38,6 @@ def _worker(rank, world, port, free, inst, ret):
     assert st["evaluations"] == 7, st      # 1 eager + 1 warm-up before the capture + 5 replays
     for a_, b_ in zip(outs, (res, jac, cost, grad)):
         assert torch.equal(a_, b_)
-    sc2 = ShardedCollocation(16, 500, 0.02, (0., 0.), inst, copy.copy(cs), engine=eng, backend="collective")   # NCCL all-gather + all-reduce
-    res2, jac2, cost2, grad2 = sc2.evaluate(fl)
-    for a_, b_, tol in ((res2, res, 1e-14), (jac2, jac, 1e-14), (grad2, grad, 1e-13)):      # two different kernels: same values, not same bits
-        assert torch.allclose(a_, b_, rtol=tol, atol=1e-16), float((a_ - b_).abs().max())
-    assert abs(float(cost2[0]) - float(cost[0])) <= 1e-13 * abs(float(cost[0]))
     # a batch larger than the co-resident grid (160 problems x 16 tiles = 2560 items; 12 blocks x 148 SMs are resident): the
     # persistent item loop of the fused kernel, every rank against its own unsharded evaluation of the same batch
     from d2d_b200.collocation import CollocationProblem
