@@ -132,24 +132,20 @@ __global__ void __launch_bounds__(kThreads) dfff_control_kernel(const d2dx_traj_
   double x[5];
   for (int k = 0; k < 5; ++k) x[k] = X[(size_t)k * B + b];
   const CareConst cc = care_const(g);
-  CareState cs = {0.0, 1.0, 1.0, 0.0, 0.0};
-  bool cold = true;
-  if (care_state) {
-    cs.C = care_state[b]; cs.S = care_state[B + b]; cs.al = care_state[2 * (size_t)B + b];
-    cs.dth = care_state[3 * (size_t)B + b]; cs.dal = care_state[4 * (size_t)B + b];
-    cold = !(cs.al > 0.0);
-  }
+  double cs[kCareState] = {};
+  if (care_state)
+    for (int k = 0; k < kCareState; ++k) cs[k] = care_state[k * (size_t)B + b];
+  bool cold = !(cs[2] > 0.0);
   int flags = 0;
   RefCtl rc;
   double u_phi, u_v;
-  make_ref(Y, a, ac[B + b], cc, cs, cold, flags, rc);
+  make_ref(Y, a, ac[B + b], cc, ArrayState{cs}, cold, flags, rc);
   feedback(rc, x, g, u_phi, u_v);
   U[b] = u_phi; U[(size_t)B + b] = u_v;
   if (Xr) { Xr[b] = rc.xr; Xr[(size_t)B + b] = rc.yr; Xr[2 * (size_t)B + b] = rc.psir; Xr[3 * (size_t)B + b] = rc.phir; Xr[4 * (size_t)B + b] = rc.var; }
   if (K) for (int k = 0; k < 6; ++k) K[(size_t)k * B + b] = rc.k[k];
   if (care_state) {
-    care_state[b] = cs.C; care_state[B + b] = cs.S; care_state[2 * (size_t)B + b] = cold ? 0.0 : cs.al;
-    care_state[3 * (size_t)B + b] = cs.dth; care_state[4 * (size_t)B + b] = cs.dal;
+    for (int k = 0; k < kCareState; ++k) care_state[k * (size_t)B + b] = (k == 2 && cold) ? 0.0 : cs[k];
   }
 }
 

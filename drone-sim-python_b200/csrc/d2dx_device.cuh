@@ -452,15 +452,28 @@ __host__ __device__ __forceinline__ int hi_word(double x) {
 #endif
 }
 
-struct CareState { double C, S, al, dth, dal; };   // solution of the previous control step and its last change
+// The Riccati warm start carried from one control step to the next, 9 doubles in the order of d2dx_rollout_out.care_state's
+// rows: the solution C, S, al of the previous step (al <= 0 only in a cold state), then the changes of theta (sines of the
+// angle steps) at steps n, n-1, n-2 and those of al.  Callers keep it where it suits them and pass an accessor st(k)
+// returning a reference to row k.
+constexpr int kCareState = D2DX_CARE_STATE_ROWS;
+struct CareSol { double C, S, al, be; };   // solution of one step; be = kappa_3's second component
+struct ArrayState {                        // the accessor over a plain array
+  double* p;
+  __host__ __device__ double& operator()(int k) const { return p[k]; }
+};
 
-struct CareConst { double sq, q3, sr1, sr2, isr1, isr2; };
+// sqrt(Q), sqrt(R) and their products as care_gain and make_ref use them (folded once on the host, not per step)
+struct CareConst { double q3, sr1, sr2, isr1, isr2, sq2, sq_isr1, sq_isr2; };
 
-__host__ __device__ __forceinline__ CareConst care_const(const d2dx_dfff_gains& g) {
+__host__ __device__ __forceinline__ CareConst care_const(double sq, double q3, double sr1, double sr2) {
   CareConst c;
-  c.sq = ::sqrt(g.q_pos); c.q3 = g.q_psi; c.sr1 = ::sqrt(g.r_phi); c.sr2 = ::sqrt(g.r_v);
-  c.isr1 = 1.0 / c.sr1; c.isr2 = 1.0 / c.sr2;
+  c.q3 = q3; c.sr1 = sr1; c.sr2 = sr2; c.isr1 = 1.0 / sr1; c.isr2 = 1.0 / sr2;
+  c.sq2 = 2.0 * sq; c.sq_isr1 = sq * c.isr1; c.sq_isr2 = sq * c.isr2;
   return c;
+}
+__host__ __device__ __forceinline__ CareConst care_const(const d2dx_dfff_gains& g) {
+  return care_const(::sqrt(g.q_pos), g.q_psi, ::sqrt(g.r_phi), ::sqrt(g.r_v));
 }
 
 struct CareStep { double k1, ba, vc2, ve, k2, q3; };   // per-control-step constants of the two residuals
@@ -479,7 +492,7 @@ __host__ __device__ __forceinline__ void care_update(double& C, double& S, doubl
   C = Cn * nrm; S = Sn * nrm; al += dal;
 }
 
-// Full Newton iteration loop (cold starts, trajectory corners, anything the two-step fast path did not finish).
+// Full Newton iteration loop (cold starts, trajectory corners, anything the straight-line step did not finish).
 struct CareRoot { double C, S, al; bool conv; };
 static __host__ __device__ __noinline__ CareRoot care_newton_loop_v(const CareStep k, double C, double S, double al, int max_it) {
   bool conv = false;
@@ -506,52 +519,68 @@ __host__ __device__ __forceinline__ bool care_newton_loop(const CareStep& k, dou
   return r.conv;
 }
 
-// Gain in the path frame.  Warm start = previous solution extrapolated by its last change (the reference moves
-// smoothly, so the start is already O(drift^2) close); then ONE Newton step and ONE chord step (same Jacobian) in
-// straight-line code, accepted when the chord step is below 3e-8 (=> error ~1e-15); otherwise the general loop.
-// Returns false when not even the loop converged.
-__host__ __device__ __forceinline__ bool care_gain(const CareConst& cc, double v, double c1, double e, CareState& st, bool cold, double* K0) {
-  const double c1q = c1 * cc.sq;                                   // c1 = sqrt(r1)/b1, e = b2 c1
-  CareStep k;
-  k.k1 = c1q * cc.isr2; k.ba = e * cc.isr2; k.vc2 = v * cc.sr2; k.ve = v * e; k.k2 = 2.0 * v * c1q; k.q3 = cc.q3;
-  // The warm path runs unconditionally and in straight-line code (a cold state -- C = 0, S = 1, al = 1 -- only produces numbers
-  // that are thrown away): its instructions share one block with the flatness / arctangent work before it, and ONE branch
-  // afterwards takes the cold start, a failed acceptance test and the restart.
-  const double C0 = st.C, S0 = st.S, al0 = st.al;
-  double C = C0, S = S0, al = al0;
-  care_update(C, S, al, st.dth, st.dal);                           // extrapolate
+// Acceptance bound of the single Newton step: |dth| and |dal| / al below 2^-23 = 1.19e-7, decided on the integer pipe (high
+// words; hi(x) < hi(y) implies x < y for positive doubles, and adding 23 << 20 to a high word multiplies by 2^23).  The error
+// the step leaves is quadratic in it: <= 1.04 |step|^2 (theta absolute, al relative) around the roots of the C5 population,
+// so <= 1.5e-14 -- and the cubic warm start is within 3e-8, so the step stays below the bound.
+constexpr int kCareStepTolHi = 0x3E800000;          // hi(2^-23)
+constexpr int kCareStepTolExp = 23 << 20;
+enum { CARE_FAILED = 0, CARE_LOOP = 1, CARE_FAST = 2 };
+
+// Gain in the path frame.  Warm start = cubic extrapolation of the previous solutions from their last three changes
+// (theta rotated by 3 (d[n] - d[n-1]) + d[n-2], al alike), which is O(dt^4) close to the new root while the reference
+// moves smoothly (<= 3e-8 on the C5 circles at dt = 0.01); then ONE Newton step in straight-line code, accepted when it
+// is below 2^-23.  Otherwise the general loop.  The solution goes to sol and, with the updated history, to st.
+// Returns CARE_FAST when the straight-line step was accepted, CARE_LOOP when the loop converged, CARE_FAILED when not
+// even the cold start did.
+template <class State>
+__host__ __device__ __forceinline__ int care_gain(const CareConst& cc, double v, double c1, double e, State&& st, bool cold, CareSol& sol) {
+  CareStep k;                                                      // c1 = sqrt(r1)/b1, e = b2 c1
+  k.k1 = c1 * cc.sq_isr2; k.ba = e * cc.isr2; k.vc2 = v * cc.sr2; k.ve = v * e; k.k2 = v * c1 * cc.sq2; k.q3 = cc.q3;
+  // The warm path runs unconditionally and in straight-line code (a cold state only produces numbers that are thrown away):
+  // its instructions share one block with the flatness / arctangent work before it, and ONE branch afterwards takes the cold
+  // start, a failed acceptance test and the restart.  The extrapolation needs only the previous step's data, so it can issue
+  // before this step's flatness work.
+  const double th1 = st(3), th2 = st(4), th3 = st(5), al1 = st(6), al2 = st(7), al3 = st(8);
+  st(4) = th1; st(5) = th2; st(7) = al1; st(8) = al2;              // age the history; this step's change goes to 3 and 6
+  // extrapolate: rotate (C, S) by the angle whose sine is the extrapolated change p (cos = 1 - p^2/2 up to p^4/8, which the
+  // Newton step's normalisation removes), as the changes were measured
+  const double p = fma(3.0, th1 - th2, th3), cp = fma(-0.5 * p, p, 1.0);
+  double C = fma(st(0), cp, -st(1) * p), S = fma(st(1), cp, st(0) * p), al = st(2) + fma(3.0, al1 - al2, al3);
   double be_, F1, F2;
   care_residual(k, C, S, al, be_, F1, F2);
   const double bt = -k.k1 * S;
   const double J11 = fma(-S, al, fma(C, be_, fma(S, bt, fma(k.ve, C, -k.vc2 * S)))), J12 = fma(S, k.ba, C);
   const double J21 = 2.0 * fma(be_, bt, -0.5 * k.k2 * C), J22 = 2.0 * fma(be_, k.ba, al);
   const double idet = rcp_f(fma(J11, J22, -J12 * J21));
-  const double i11 = J22 * idet, i12 = -J12 * idet, i21 = -J21 * idet, i22 = J11 * idet;   // J^-1
-  double dth = -fma(i11, F1, i12 * F2), dal = -fma(i21, F1, i22 * F2);
+  const double dth = fma(J12, F2, -F1 * J22) * idet, dal = fma(J21, F1, -J11 * F2) * idet;
   care_update(C, S, al, dth, dal);                                 // Newton step
-  care_residual(k, C, S, al, be_, F1, F2);
-  dth = -fma(i11, F1, i12 * F2); dal = -fma(i21, F1, i22 * F2);
-  care_update(C, S, al, dth, dal);                                 // chord step
-  // accept when the chord step is tiny AND the root is on the stabilising branch (S > 0, al > 0 there: kappa_2's
+  // accept when the step is tiny AND the root is on the stabilising branch (S > 0, al > 0 there: kappa_2's
   // first component and K_13 are positive for every v, b1 > 0)
-  // (sign tests and the fixed threshold on the integer pipe: hi word of 3e-8 = 0x3E601B2B; S, al > 0 <=> sign bit clear, not zero)
-  bool ok = !cold && (hi_word(dth) & 0x7fffffff) < 0x3E601B2B && fabs(dal) < 3e-8 * fabs(al) && hi_word(S) > 0 && hi_word(al) > 0;
-  if (!ok) {
-    if (!cold) {                                                   // corner of the reference, big jump: iterate from the
-      C = C0; S = S0; al = al0;                                    // previous solution, not from the failed extrapolation
-      ok = care_newton_loop(k, C, S, al, 40) && S > 0.0 && al > 0.0;
+  // (sign tests and the fixed threshold on the integer pipe; S, al > 0 <=> sign bit clear, not zero)
+  const int hal = hi_word(al);
+  int res = (!cold && (hi_word(dth) & 0x7fffffff) < kCareStepTolHi && (hi_word(dal) & 0x7fffffff) + kCareStepTolExp < hal &&
+             hi_word(S) > 0 && hal > 0) ? CARE_FAST : CARE_FAILED;
+  if (res == CARE_FAILED) {
+    if (!cold) {                                                   // corner of the reference, big jump, history still building
+      C = st(0); S = st(1); al = st(2);                            // up: iterate from the previous solution, not from the extrapolation
+      if (care_newton_loop(k, C, S, al, 40) && S > 0.0 && al > 0.0) res = CARE_LOOP;
     }
-    if (!ok) { C = 0.0; S = 1.0; al = sqrt_f(cc.q3 + k.k2); ok = care_newton_loop(k, C, S, al, 60); }   // cold start: decoupled (b2 = 0) solution
+    if (res == CARE_FAILED) {                                      // cold start: decoupled (b2 = 0) solution
+      C = 0.0; S = 1.0; al = sqrt_f(cc.q3 + k.k2);
+      if (care_newton_loop(k, C, S, al, 60)) res = CARE_LOOP;
+    }
   }
   // change over this control step (angle from the cross product of the unit vectors); only a small, smooth change is worth
-  // extrapolating -- and none after a cold start
-  st.dth = fma(C0, S, -S0 * C); st.dal = al - al0;
-  if (cold || !((hi_word(st.dth) & 0x7fffffff) < 0x3F947AE1 && fabs(st.dal) < 0.02 * al)) { st.dth = 0.0; st.dal = 0.0; }   // hi(0.02)
-  st.C = C; st.S = S; st.al = al;
-  const double be = fma(k.k1, C, k.ba * al);
-  K0[0] = cc.sq * C * cc.isr1; K0[1] = cc.sq * S * cc.isr1; K0[2] = al * cc.isr1;
-  K0[3] = cc.sq * S * cc.isr2; K0[4] = -cc.sq * C * cc.isr2; K0[5] = be * cc.isr2;
-  return ok;
+  // extrapolating -- and none after a cold start: the history restarts from zero and the next three steps take the loop
+  const double nth = fma(st(0), S, -st(1) * C), nal = al - st(2);
+  // (|nth| < 0.02 and |nal| < al / 64 on the integer pipe; a negative al fails the second test)
+  const bool keep = !cold && (hi_word(nth) & 0x7fffffff) < 0x3F947AE1 && (hi_word(nal) & 0x7fffffff) + (6 << 20) < hi_word(al);
+  st(0) = C; st(1) = S; st(2) = al;
+  st(3) = keep ? nth : 0.0; st(6) = keep ? nal : 0.0;
+  if (!keep) { st(4) = 0.0; st(5) = 0.0; st(7) = 0.0; st(8) = 0.0; }
+  sol.C = C; sol.S = S; sol.al = al; sol.be = fma(k.k1, C, k.ba * al);
+  return res;
 }
 
 // DFFFController.get (d2d/guidance.py:62-91) split in two.  Everything up to the gain depends on the reference
@@ -559,7 +588,8 @@ __host__ __device__ __forceinline__ bool care_gain(const CareConst& cc, double v
 // interleaved with the RK4 stages of the current step (two independent dependency chains per thread).
 struct RefCtl { double xr, yr, psir, phir, var, uphi, uv, k[6]; };   // reference state, feed-forward input, K1 = K' T (2x3)
 
-__device__ __forceinline__ void make_ref(const FlatOut& Y, const AcPar& a, double tau_v, const CareConst& cc, CareState& cs,
+template <class State>
+__device__ __forceinline__ void make_ref(const FlatOut& Y, const AcPar& a, double tau_v, const CareConst& cc, State&& care,
                                          bool& cold, int& flags, RefCtl& r) {
   FlatState fr;
   flatness(Y, a.wx, a.wy, tau_v, fr);
@@ -568,16 +598,15 @@ __device__ __forceinline__ void make_ref(const FlatOut& Y, const AcPar& a, doubl
   const double z2 = fr.z * fr.z;
   const double c1 = cc.sr1 * (2.0 + z2) * rcp_f(kG * fr.inv_va * (1.0 + z2));
   const double e = kG * fr.inv_va * fr.inv_va * fr.z * c1;
-  double K0[6];
-  if (care_gain(cc, fr.va, c1, e, cs, cold, K0)) cold = false;
+  CareSol cs;
+  if (care_gain(cc, fr.va, c1, e, care, cold, cs) != CARE_FAILED) cold = false;
   else { flags |= 2; cold = true; }
   r.xr = fr.x; r.yr = fr.y; r.psir = fr.psi; r.phir = fr.phi; r.var = fr.va; r.uphi = fr.u_phi; r.uv = fr.u_v;
-#pragma unroll
-  for (int m = 0; m < 2; ++m) {                                  // K1 = K' T,  T = rot(-psi_ref) (+) 1
-    r.k[3 * m + 0] = K0[3 * m] * fr.cpsi - K0[3 * m + 1] * fr.spsi;
-    r.k[3 * m + 1] = K0[3 * m] * fr.spsi + K0[3 * m + 1] * fr.cpsi;
-    r.k[3 * m + 2] = K0[3 * m + 2];
-  }
+  // K1 = K' T,  T = rot(-psi_ref) (+) 1,  K' = [[sqrt(q) (C, S), al] / sqrt(r1) ; [sqrt(q) (S, -C), be] / sqrt(r2)]:
+  // both rows rotate the same unit vector (C, S)
+  const double Cw = fma(cs.C, fr.cpsi, -cs.S * fr.spsi), Sw = fma(cs.C, fr.spsi, cs.S * fr.cpsi);
+  r.k[0] = cc.sq_isr1 * Cw; r.k[1] = cc.sq_isr1 * Sw; r.k[2] = cs.al * cc.isr1;
+  r.k[3] = cc.sq_isr2 * Sw; r.k[4] = -cc.sq_isr2 * Cw; r.k[5] = cs.be * cc.isr2;
 }
 
 // the state-dependent rest: error, wrap, saturations, feedback (d2d/guidance.py:67-70,85-88)

@@ -113,12 +113,12 @@ __host__ __device__ inline bool lqr5_gain(const Lqr5Par& P, double sr1, double s
     if (ok) st = w;
   }
   if (!ok) {                                                         // cold: the 3-state gain as the first guess
-    CareConst cc; cc.sq = P.sq; cc.q3 = P.q3; cc.sr1 = sr1; cc.sr2 = sr2; cc.isr1 = 1.0 / sr1; cc.isr2 = 1.0 / sr2;
-    CareState c3 = {0.0, 1.0, 1.0, 0.0, 0.0};
-    double K0[6];
+    const CareConst cc = care_const(P.sq, P.q3, sr1, sr2);
+    double s3[kCareState] = {};
+    CareSol c3;
     const double c1 = sr1 * rcp_f(P.a), e = P.b * c1;
-    care_gain(cc, P.v, c1, e, c3, true, K0);
-    const double al3 = K0[2] * sr1, be3 = K0[5] * sr2;
+    care_gain(cc, P.v, c1, e, ArrayState{s3}, true, c3);
+    const double al3 = c3.al, be3 = c3.be;
     st.C = c3.C; st.S = c3.S;
     st.p23 = P.s1 * al3; st.p24 = P.s2 * be3;
     st.p33 = tau_phi * (P.a * st.p23 + 0.5 * P.q4);

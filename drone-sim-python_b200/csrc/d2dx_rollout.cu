@@ -93,13 +93,11 @@ __global__ void __launch_bounds__(kRolloutThreads, D2DX_ROLLOUT_MIN_BLOCKS) roll
   for (int k = 0; k < 5; ++k) X[k] = a.s.X0[(size_t)k * B + b];
 
   const CareConst& cc = a.cc;
-  CareState cs = {0.0, 1.0, 1.0, 0.0, 0.0};
-  bool cold = true;
-  if (a.o.care_state) {
-    cs.C = a.o.care_state[b]; cs.S = a.o.care_state[B + b]; cs.al = a.o.care_state[2 * (size_t)B + b];
-    cs.dth = a.o.care_state[3 * (size_t)B + b]; cs.dal = a.o.care_state[4 * (size_t)B + b];
-    cold = !(cs.al > 0.0);
-  }
+  // the Riccati warm start (care_gain's state rows) in registers: a shared-memory column per thread measured 2.7 % slower
+  double care[kCareState];
+#pragma unroll
+  for (int k = 0; k < kCareState; ++k) care[k] = a.o.care_state ? a.o.care_state[k * (size_t)B + b] : 0.0;
+  bool cold = !(care[2] > 0.0);                                   // no state, or zeros: cold
   int flags = 0;
   double sum_sq = 0.0, max_sq = 0.0;
 
@@ -124,7 +122,7 @@ __global__ void __launch_bounds__(kRolloutThreads, D2DX_ROLLOUT_MIN_BLOCKS) roll
       }
       segment_eval<false>(seg_type, P, te, Y, &tt);
     }
-    make_ref(Y, load_ac(), spar[D2DX_SEG_NPAR + 4][tid], cc, cs, cold, flags, r);
+    make_ref(Y, load_ac(), spar[D2DX_SEG_NPAR + 4][tid], cc, ArrayState{care}, cold, flags, r);
   };
 
   const int log_every = a.o.log_every > 0 ? a.o.log_every : 1;
@@ -183,9 +181,8 @@ __global__ void __launch_bounds__(kRolloutThreads, D2DX_ROLLOUT_MIN_BLOCKS) roll
     if (a.o.max_err) a.o.max_err[b] = fmax(a.o.max_err[b], sqrt(max_sq));
     if (a.o.flags) a.o.flags[b] |= flags;
     if (a.o.care_state) {
-      a.o.care_state[b] = cs.C; a.o.care_state[B + b] = cs.S;
-      a.o.care_state[2 * (size_t)B + b] = cold ? 0.0 : cs.al;
-      a.o.care_state[3 * (size_t)B + b] = cs.dth; a.o.care_state[4 * (size_t)B + b] = cs.dal;
+#pragma unroll
+      for (int k = 0; k < kCareState; ++k) a.o.care_state[k * (size_t)B + b] = (k == 2 && cold) ? 0.0 : care[k];
     }
   }
   if (a.o.pop_stats) {                 // population reductions: warp shuffles, one atomic per warp

@@ -10,19 +10,35 @@ using namespace d2dx;
 
 extern "C" {
 
-// LQR gain of DFFFController.get (d2d/guidance.py:78-82) in the path frame (psi_ref = 0) at reference speed v and bank phi:
-// K0[6] = row-major 2x3.  state5 (in/out): C, S, al, dth, dal; cold != 0 ignores it.  Returns 1 when converged.
-int d2dx_host_care_gain(const double* qr4 /* q_pos, q_psi, r_phi, r_v */, double v, double phi, int cold, double* state5, double* K0) {
+static int care_gain_host(const double* qr4, double v, double phi, int cold, double* state9, double* K0) {
   d2dx_dfff_gains g;
   g.q_pos = qr4[0]; g.q_psi = qr4[1]; g.r_phi = qr4[2]; g.r_v = qr4[3];
   const CareConst cc = care_const(g);
   const double z = tan(phi), z2 = z * z, inv_va = 1.0 / v;
   const double c1 = cc.sr1 * (2.0 + z2) * rcp_f(kG * inv_va * (1.0 + z2));   // as make_ref forms them
   const double e = kG * inv_va * inv_va * z * c1;
-  CareState st = {state5[0], state5[1], state5[2], state5[3], state5[4]};
-  const bool ok = care_gain(cc, v, c1, e, st, cold != 0, K0);
-  state5[0] = st.C; state5[1] = st.S; state5[2] = st.al; state5[3] = st.dth; state5[4] = st.dal;
-  return ok ? 1 : 0;
+  CareSol sol;
+  const int res = care_gain(cc, v, c1, e, ArrayState{state9}, cold != 0, sol);
+  K0[0] = cc.sq_isr1 * sol.C; K0[1] = cc.sq_isr1 * sol.S; K0[2] = sol.al * cc.isr1;   // make_ref's K1 at psi_ref = 0
+  K0[3] = cc.sq_isr2 * sol.S; K0[4] = -cc.sq_isr2 * sol.C; K0[5] = sol.be * cc.isr2;
+  return res;
+}
+
+// LQR gain of DFFFController.get (d2d/guidance.py:78-82) in the path frame (psi_ref = 0) at reference speed v and bank phi:
+// K0[6] = row-major 2x3.  state9 (in/out): C, S, al, then the changes of theta at steps n, n-1, n-2 and those of al
+// (d2dx_rollout_out.care_state's rows); cold != 0 ignores it.  Returns 2 when the straight-line step was accepted, 1 when
+// the fallback loop converged, 0 when nothing did.
+int d2dx_host_care_gain9(const double* qr4 /* q_pos, q_psi, r_phi, r_v */, double v, double phi, int cold, double* state9, double* K0) {
+  return care_gain_host(qr4, v, phi, cold, state9, K0);
+}
+
+// The same with a 5-double state: C, S, al and the LAST change of theta and al only; the two older changes are taken equal
+// to it, which makes the warm start a linear extrapolation.  Returns 1 when converged.
+int d2dx_host_care_gain(const double* qr4, double v, double phi, int cold, double* state5, double* K0) {
+  double s9[9] = {state5[0], state5[1], state5[2], state5[3], state5[3], state5[3], state5[4], state5[4], state5[4]};
+  const int res = care_gain_host(qr4, v, phi, cold, s9, K0);
+  state5[0] = s9[0]; state5[1] = s9[1]; state5[2] = s9[2]; state5[3] = s9[3]; state5[4] = s9[6];
+  return res != CARE_FAILED ? 1 : 0;
 }
 
 // 5-state LQR gain of DiffController.ComputeGain (Controllers.py:159-186) in the path frame: Kp[10] = row-major 2x5.

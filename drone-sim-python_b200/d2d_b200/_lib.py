@@ -15,6 +15,7 @@ EVAL_RESIDUAL, EVAL_JAC, EVAL_COST, EVAL_GRAD = 1, 2, 4, 8
 EVAL_ALL = 15
 MAX_OBSTACLES = 16
 PEER_MAX_WORLD, IPC_HANDLE_BYTES = 16, 64
+CARE_STATE_ROWS = 9    # D2DX_CARE_STATE_ROWS: rows of the Riccati warm start (care_state)
 
 c_dp = C.c_void_p      # device pointers travel as integers
 

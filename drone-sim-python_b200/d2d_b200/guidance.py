@@ -64,7 +64,8 @@ class DFFFController:
         eng = get_engine()
         if self._table is None:
             self._table = eng.table(ddt.pack([self.traj]))
-            self._care = eng.zeros(5, 1)
+            from . import _lib
+            self._care = eng.zeros(_lib.CARE_STATE_ROWS, 1)
         W = np.asarray(self.wind.sample(t, None), dtype=np.float64).reshape(2, 1)
         acd = eng.to_device(np.array([[self.ac.tau_phi], [self.ac.tau_v]]))
         Xd = eng.to_device(np.asarray(X, dtype=np.float64).reshape(5, 1))

@@ -106,7 +106,8 @@ def rollout(time, trajs, wind, X0, perts=None, tau_phi=0.01, tau_v=1., nsub=1, l
     K_log = eng.empty(n_rows, 6, B) if (log_ref and return_log) else None
     sum_sq, max_err = eng.zeros(B), eng.zeros(B)
     flags = eng.zeros(B, dtype=torch.int32)
-    care = eng.zeros(5, B)
+    from . import _lib
+    care = eng.zeros(_lib.CARE_STATE_ROWS, B)
     pop = eng.zeros(2)
     X_final = eng.empty(5, B)
     chunk = chunk_steps or (T - 1)
@@ -304,7 +305,7 @@ class MonteCarloRollout:
         self.d_Ulog = eng.empty(self.n_rows, 2, B) if log_u else None
         self.d_Xf, self.d_Xa, self.d_Xb = eng.empty(5, B), eng.empty(5, B), eng.empty(5, B)
         self.d_ss, self.d_mx, self.d_flags = eng.zeros(B), eng.zeros(B), eng.zeros(B, dtype=torch.int32)
-        self.d_care, self.d_pop = eng.zeros(5, B), eng.zeros(2)
+        self.d_care, self.d_pop = eng.zeros(_lib.CARE_STATE_ROWS, B), eng.zeros(2)
         # chunk boundaries aligned to the log stride
         steps = self.T - 1
         per = max(self.log_every, ((steps + n_chunks - 1) // n_chunks + self.log_every - 1) // self.log_every * self.log_every)

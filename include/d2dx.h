@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define D2DX_VERSION 103
+#define D2DX_VERSION 104
 
 enum { D2DX_OK = 0, D2DX_EINVAL = 1, D2DX_ECUDA = 2, D2DX_EUNSUPPORTED = 3 };
 
@@ -122,9 +122,13 @@ typedef struct {
 } d2dx_dfff_gains;
 int d2dx_dfff_default_gains(d2dx_dfff_gains* g_host);
 
+/* Rows of the Riccati warm start (care_state): the previous solution (C, S, alpha; alpha = 0 when cold), then the changes of
+ * theta and of alpha over the last three control steps, from which the next solution is extrapolated. */
+#define D2DX_CARE_STATE_ROWS 9
+
 /* DFFFController.get(X, t), d2d/guidance.py:62-91, for B aircraft at one time `t`.
  * Outputs U[2][B]; optional Xr[5][B], K[6][B] (row-major 2x3 = K[:, :3]; K[:, 3:] is zero).
- * care_state[5][B] (optional, in/out, zero-initialised) warm-starts the Riccati solve. */
+ * care_state[D2DX_CARE_STATE_ROWS][B] (optional, in/out, zero-initialised) warm-starts the Riccati solve. */
 int d2dx_dfff_control(d2dx_handle* h, const d2dx_traj_table* tt, const double* X, double t,
                       const double* W, const double* ac, const d2dx_dfff_gains* gains_host,
                       double* U, double* Xr, double* K, double* care_state, void* stream);
@@ -155,7 +159,7 @@ typedef struct {
   double* sum_sq_err;        /* [B] or NULL  += sum_i |X[i,:2]-Xr[i,:2]|^2 over this call        */
   double* max_err;           /* [B] or NULL  = max(previous, max_i |X[i,:2]-Xr[i,:2]|)           */
   int32_t* flags;            /* [B] or NULL  |= 1 non-finite state seen, 2 Riccati not converged */
-  double* care_state;        /* [5][B] or NULL  Riccati warm start carried between calls (zeros = cold) */
+  double* care_state;        /* [D2DX_CARE_STATE_ROWS][B] or NULL  Riccati warm start carried between calls (zeros = cold) */
   double* pop_stats;         /* [2] or NULL  += sum over scenarios of sum_sq_err; max of max_err */
 } d2dx_rollout_out;
 
