@@ -7,28 +7,13 @@ namespace d2dx {
 constexpr int kDdpWarps = 4;                       // problems (= warps) per block
 constexpr int kDdpSlot = 24;                       // doubles of staging per lane
 
-// fills the solver's problem description from the collocation problem + bounds + box
-__host__ inline int ddp_problem_from(const d2dx_colloc_problem* p, const double* bounds, const double* box, DdpProblem& P) {
-  if (!p || p->n_ac != 1 || p->N < 2 || !(p->h > 0) || !bounds) return 1;
-  const double sN = p->obj_scale / p->N, nin = sN / (p->in_div >= 1 ? p->in_div : 1);
-  P.N = p->N; P.h = p->h; P.wx = p->wind[0]; P.wy = p->wind[1];
-  P.vsp = p->vsp; P.kv = p->kvel * nin; P.kb = p->kbank * nin;
-  const bool obs = (p->kobs == p->kobs) && p->kobs != 0.0 && p->n_obs > 0;
-  P.kobs = obs ? p->kobs * sN : 0.0; P.n_obs = obs ? p->n_obs : 0; P.obs_kind = p->obs_kind;
-  for (int o = 0; o < P.n_obs; ++o) { P.obs[o][0] = p->obs[o][0]; P.obs[o][1] = p->obs[o][1]; P.obs[o][2] = p->obs[o][2]; }
-  P.phi_lo = bounds[0]; P.phi_hi = bounds[1]; P.v_lo = bounds[2]; P.v_hi = bounds[3];
-  P.has_box = box != nullptr;
-  if (box) { P.x_lo = box[0]; P.x_hi = box[1]; P.y_lo = box[2]; P.y_hi = box[3]; P.w_box = box[4] * sN; }
-  else { P.x_lo = P.y_lo = -1e300; P.x_hi = P.y_hi = 1e300; P.w_box = 0.0; }
-  return (P.phi_lo < P.phi_hi && P.v_lo < P.v_hi && P.v_lo > 0.0) ? 0 : 1;
-}
-
 // Sweeps of ONE problem by ONE warp.  The recursion over the nodes is sequential (lane 0 carries it), but everything around it
 // is not: per chunk of 32 nodes the lanes load the trajectory coalesced, evaluate the transcendental functions, the obstacle
 // exponentials and the costs of their node in parallel and stage the results in shared memory; lane 0 then runs the node
 // algebra from shared memory (about 250 fp64 instructions per node, no memory latency, no libm call in the dependent chain),
 // and the lanes write the gains / the new trajectory back coalesced.  Same node functions as the serial host sweeps.
 struct DdpWarp {
+  static constexpr int kMaxCon = 3;
   const DdpProblem& P;
   DdpWork W;                                        // stride 1: this problem's arrays are contiguous
   const double* zt;
@@ -44,6 +29,7 @@ struct DdpWarp {
     return __shfl_sync(0xffffffffu, s, 0) != 0;
   }
   __device__ void count_solved() { if (lane == 0) atomicAdd(solved, 1); }
+  __device__ int n_con() const { return 3; }
 
   __device__ DdpSweep backward(const double* lam, double rho, double mu, int reg_mode) {
     const int N = P.N;

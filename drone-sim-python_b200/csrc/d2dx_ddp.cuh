@@ -33,6 +33,22 @@ struct DdpProblem {
   double x_lo, x_hi, y_lo, y_hi, w_box;   // w_box = weight * obj_scale / N
 };
 
+// fills the solver's problem description from the collocation problem + bounds + box (every aircraft shares them)
+__host__ inline int ddp_problem_from(const d2dx_colloc_problem* p, const double* bounds, const double* box, DdpProblem& P, int max_ac = 1) {
+  if (!p || p->n_ac < 1 || p->n_ac > max_ac || p->N < 2 || !(p->h > 0) || !bounds) return 1;
+  const double sN = p->obj_scale / p->N, nin = sN / (p->in_div >= 1 ? p->in_div : 1);
+  P.N = p->N; P.h = p->h; P.wx = p->wind[0]; P.wy = p->wind[1];
+  P.vsp = p->vsp; P.kv = p->kvel * nin; P.kb = p->kbank * nin;
+  const bool obs = (p->kobs == p->kobs) && p->kobs != 0.0 && p->n_obs > 0;
+  P.kobs = obs ? p->kobs * sN : 0.0; P.n_obs = obs ? p->n_obs : 0; P.obs_kind = p->obs_kind;
+  for (int o = 0; o < P.n_obs; ++o) { P.obs[o][0] = p->obs[o][0]; P.obs[o][1] = p->obs[o][1]; P.obs[o][2] = p->obs[o][2]; }
+  P.phi_lo = bounds[0]; P.phi_hi = bounds[1]; P.v_lo = bounds[2]; P.v_hi = bounds[3];
+  P.has_box = box != nullptr;
+  if (box) { P.x_lo = box[0]; P.x_hi = box[1]; P.y_lo = box[2]; P.y_hi = box[3]; P.w_box = box[4] * sN; }
+  else { P.x_lo = P.y_lo = -1e300; P.x_hi = P.y_hi = 1e300; P.w_box = 0.0; }
+  return (P.phi_lo < P.phi_hi && P.v_lo < P.v_hi && P.v_lo > 0.0) ? 0 : 1;
+}
+
 struct DdpWork {                   // element (k, node) of an array lives at base[(k * N + node) * stride]
   double *u, *z, *un, *zn, *k, *K;
   long stride;
@@ -247,6 +263,7 @@ __host__ __device__ __forceinline__ void ddp_forward_node(const DdpProblem& P, d
 
 // ---- serial sweeps over one problem's arrays (host build; also the reference of the warp-cooperative device sweeps) ----
 struct DdpSerial {
+  static constexpr int kMaxCon = 3;
   const DdpProblem& P;
   DdpWork W;
   const double* zt;
@@ -303,6 +320,7 @@ struct DdpSerial {
     double* t = W.u; W.u = W.un; W.un = t;
     t = W.z; W.z = W.zn; W.zn = t;
   }
+  __host__ __device__ int n_con() const { return 3; }
   __host__ __device__ bool enough_solved() const { return false; }
   __host__ __device__ void count_solved() {}
   // terminal error of the current trajectory
@@ -330,9 +348,13 @@ struct DdpResult { int flag, iterations, outer, swaps; double cost, cmax, lagr, 
 
 // The solver: augmented-Lagrangian loop around regularised second-order sweeps.  `S` supplies the sweeps over one problem's
 // arrays (DdpSerial on the host, the warp-cooperative DdpWarp in d2dx_ddp.cu); every decision below is a scalar one.
+// S::kMaxCon bounds the number of terminal conditions S::n_con() (3 per aircraft).  lam_out (optional): the multipliers of the last
+// inner loop, the ones the returned trajectory minimises the augmented Lagrangian for.
 template <typename S>
-__host__ __device__ inline DdpResult ddp_solve(S& sw_, const double* z0, const d2dx_ddp_options& o) {
-  double lam[3] = {0.0, 0.0, 0.0}, rho = o.rho0, mu = o.mu0, dmu = 1.0;
+__host__ __device__ inline DdpResult ddp_solve(S& sw_, const double* z0, const d2dx_ddp_options& o, double* lam_out = nullptr) {
+  const int nc = sw_.n_con();
+  double lam[S::kMaxCon], rho = o.rho0, mu = o.mu0, dmu = 1.0;
+  for (int k = 0; k < nc; ++k) lam[k] = 0.0;
   sw_.prepare(z0);
   double cost, cmax, J = sw_.forward(0.0, lam, rho, cost, cmax);     // zero gains: the rollout of the start inputs
   sw_.accept();
@@ -341,6 +363,7 @@ __host__ __device__ inline DdpResult ddp_solve(S& sw_, const double* z0, const d
   int it = 0;
   bool stop = false;
   for (int outer = 0; outer < o.max_outer && it < o.max_iter && !stop; ++outer) {
+    if (lam_out) for (int k = 0; k < nc; ++k) lam_out[k] = lam[k];
     bool converged = false;
     for (int inner = 0; inner < o.max_inner && it < o.max_iter; ++inner, ++it) {
       if (sw_.enough_solved()) { stop = true; break; }     // multi-start: enough other starts of the launch have converged
@@ -381,13 +404,16 @@ __host__ __device__ inline DdpResult ddp_solve(S& sw_, const double* z0, const d
     res.outer = outer + 1;
     if (cmax < o.ctol && converged) { res.flag = 2; sw_.count_solved(); break; }
     // multiplier / penalty update (the rule of the first-order driver: grow rho when the violation did not fall to a quarter)
-    double c[3];
+    double c[S::kMaxCon];
     sw_.terminal_error(c);
-    lam[0] += rho * c[0]; lam[1] += rho * c[1]; lam[2] += rho * c[2];
+    for (int k = 0; k < nc; ++k) lam[k] += rho * c[k];
     if (cmax > 0.25 * c_prev || outer == 0) rho = fmin(rho * o.rho_growth, o.rho_max);
     c_prev = cmax;
     mu = o.mu0; dmu = 1.0;
-    J = cost + lam[0] * c[0] + lam[1] * c[1] + lam[2] * c[2] + 0.5 * rho * (c[0] * c[0] + c[1] * c[1] + c[2] * c[2]);
+    J = cost;
+    double cc = 0.0;
+    for (int k = 0; k < nc; ++k) { J += lam[k] * c[k]; cc += c[k] * c[k]; }
+    J += 0.5 * rho * cc;
   }
   if (res.flag != 2 && !stop && cmax < o.ctol) res.flag = 4;       // feasible, but the sweep budget ran out before the cost settled
   res.iterations = it; res.cost = cost; res.cmax = cmax; res.lagr = J; res.mu = mu; res.rho = rho;

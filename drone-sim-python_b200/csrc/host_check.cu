@@ -1,9 +1,10 @@
-// Host instances of the engine's Riccati reductions (test infrastructure, not part of libd2dx.so): the SAME source the
-// kernels inline -- care_gain (d2dx_device.cuh) and lqr5_gain (d2dx_lqr5.cuh) -- compiled for the CPU, so that
-// tests/test_care_math.py can check them against scipy.linalg.solve_continuous_are without a GPU.
+// Host instances of the engine's Riccati reductions and planner solvers (test infrastructure, not part of libd2dx.so): the SAME
+// source the kernels inline -- care_gain (d2dx_device.cuh), lqr5_gain (d2dx_lqr5.cuh), the DDP solvers (d2dx_ddp.cuh,
+// d2dx_ddp_multi.cuh) -- compiled for the CPU, so that tests/test_care_math.py, test_ddp_cpu.py and test_ddp_multi_cpu.py can
+// check them without a GPU.
 #include <vector>
 
-#include "d2dx_ddp.cuh"
+#include "d2dx_ddp_multi.cuh"
 #include "d2dx_lqr5.cuh"
 
 using namespace d2dx;
@@ -59,6 +60,14 @@ int d2dx_host_lqr5_gain(const double* q5, const double* r2, double v, double phi
   return ok ? 1 : 0;
 }
 
+static d2dx_ddp_options options_or_default(const d2dx_ddp_options* o) {
+  d2dx_ddp_options opt;
+  if (o) return *o;
+  opt.max_iter = 400; opt.max_outer = 30; opt.max_inner = 40; opt.ls_max = 12; opt.ctol = 1e-8; opt.rel_tol = 1e-10; opt.abs_tol = 1e-14;
+  opt.rho0 = 10.0; opt.rho_growth = 10.0; opt.rho_max = 1e8; opt.mu0 = 1e-6; opt.mu_min = 1e-8; opt.mu_max = 1e10; opt.mu_factor = 1.6; opt.reg_mode = 0; opt.min_solved = 0;
+  return opt;
+}
+
 // The planner's second-order solver (d2dx_ddp.cuh) for ONE problem on the CPU: the code of ddp_solve_kernel's thread.
 // prob9: N, h, wx, wy, vsp, kv, kb, kobs, obs_kind (weights already normalised as DdpProblem wants them); obs[n_obs][3];
 // bounds4; box5 or NULL (x_lo, x_hi, y_lo, y_hi, w_box normalised); z0[3], zt[3]; u[2][N] in/out; xs[3][N] out; info[8] out.
@@ -78,12 +87,7 @@ int d2dx_host_ddp_solve(const double* prob9, int n_obs, const double* obs, const
   W.N = N; W.stride = 1;
   W.u = work.data(); W.z = W.u + 2 * N; W.un = W.z + 3 * N; W.zn = W.un + 2 * N; W.k = W.zn + 3 * N; W.K = W.k + 2 * N;
   for (int i = 0; i < 2 * N; ++i) W.u[i] = u[i];
-  d2dx_ddp_options opt;
-  if (o) opt = *o;
-  else {
-    opt.max_iter = 400; opt.max_outer = 30; opt.max_inner = 40; opt.ls_max = 12; opt.ctol = 1e-8; opt.rel_tol = 1e-10; opt.abs_tol = 1e-14;
-    opt.rho0 = 10.0; opt.rho_growth = 10.0; opt.rho_max = 1e8; opt.mu0 = 1e-6; opt.mu_min = 1e-8; opt.mu_max = 1e10; opt.mu_factor = 1.6; opt.reg_mode = 0; opt.min_solved = 0;
-  }
+  const d2dx_ddp_options opt = options_or_default(o);
   DdpSerial sweeps(P, W, zt);
   const DdpResult r = ddp_solve(sweeps, z0, opt);
   const double* us = (r.swaps & 1) ? W.un : W.u;
@@ -92,6 +96,50 @@ int d2dx_host_ddp_solve(const double* prob9, int n_obs, const double* obs, const
   for (int i = 0; i < 3 * N; ++i) xs[i] = zs[i];
   info[0] = r.flag; info[1] = r.iterations; info[2] = r.outer; info[3] = r.cost; info[4] = r.cmax; info[5] = r.lagr; info[6] = r.mu; info[7] = r.rho;
   return 0;
+}
+
+// The coupled multi-aircraft solver (d2dx_ddp_multi.cuh) for ONE problem on the CPU, with the arguments of d2dx_ddp_multi_solve for
+// P = 1: p0, p1 [3][n_ac]; u [2][n_ac][N] in/out; xs [3][n_ac][N] out; info[8] out; lam [3][n_ac] out or NULL.  Returns 1 for a
+// request d2dx_ddp_multi_solve refuses.
+int d2dx_host_ddp_multi_solve(const d2dx_colloc_problem* p, const double* bounds4, const double* box5, const double* p0, const double* p1,
+                              const d2dx_ddp_options* o, double* u, double* xs, double* info, double* lam) {
+  DdpmProblem M;
+  const d2dx_ddp_options opt = options_or_default(o);
+  if (ddpm_problem_from(p, bounds4, box5, M) || (opt.reg_mode != 0 && M.n > 1)) return 1;
+  const int n = M.n, N = M.a.N;
+  std::vector<double> work(DdpmWork::doubles(n, N)), scratch(DdpmNode::doubles(n)), pre(n * kDdpPre + 3 * n);
+  std::vector<int> iscratch(DdpmNode::ints(n));
+  DdpmWork W;
+  W.carve(work.data(), n, N);
+  for (int j = 0; j < 2; ++j)
+    for (int a = 0; a < n; ++a)
+      for (int i = 0; i < N; ++i) W.u[(long)i * 2 * n + 2 * a + j] = u[((long)j * n + a) * N + i];
+  double z0[3 * kDdpmMaxAc], zt[3 * kDdpmMaxAc], lm[3 * kDdpmMaxAc];
+  for (int k = 0; k < 3; ++k)
+    for (int a = 0; a < n; ++a) { z0[3 * a + k] = p0[k * n + a]; zt[3 * a + k] = p1[k * n + a]; }
+  DdpmSerial sweeps(M, W, zt, scratch.data(), iscratch.data(), pre.data());
+  const DdpResult r = ddp_solve(sweeps, z0, opt, lm);
+  const double* us = (r.swaps & 1) ? W.un : W.u;
+  const double* zs = (r.swaps & 1) ? W.zn : W.z;
+  for (int a = 0; a < n; ++a)
+    for (int i = 0; i < N; ++i) {
+      for (int j = 0; j < 2; ++j) u[((long)j * n + a) * N + i] = us[(long)i * 2 * n + 2 * a + j];
+      for (int k = 0; k < 3; ++k) xs[((long)k * n + a) * N + i] = zs[(long)i * 3 * n + 3 * a + k];
+    }
+  if (lam)
+    for (int k = 0; k < 3; ++k)
+      for (int a = 0; a < n; ++a) lam[k * n + a] = lm[3 * a + k];
+  info[0] = r.flag; info[1] = r.iterations; info[2] = r.outer; info[3] = r.cost; info[4] = r.cmax; info[5] = r.lagr; info[6] = r.mu; info[7] = r.rho;
+  return 0;
+}
+
+// The box QP of a node of the coupled solver: minimiser x[n] of 1/2 x^T H x + g^T x over lo <= x <= hi (H[n][n] row-major, positive
+// definite, n <= 20), free[n] = 1 where the component is not held at a bound.  Returns 1 when a free block was not definite.
+int d2dx_host_box_qp(int n, const double* H, const double* g, const double* lo, const double* hi, double* x, int* free_) {
+  if (n < 1 || n > 2 * kDdpmMaxAc) return 1;
+  std::vector<double> L((size_t)n * n);
+  int fi[2 * kDdpmMaxAc], nf;
+  return ddpm_box_qp(n, H, n, g, lo, hi, x, free_, fi, nf, L.data()) ? 0 : 1;
 }
 
 }  // extern "C"

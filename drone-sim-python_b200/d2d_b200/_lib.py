@@ -158,6 +158,8 @@ def _load():
         "d2dx_ddp_default_options": (C.c_int, [P(DdpOptions)]),
         "d2dx_ddp_work_size": (i64, [i32, i32]),
         "d2dx_ddp_solve": (C.c_int, [H, P(CollocProblem), i32, P(dbl), P(dbl), c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, P(DdpOptions), c_dp]),
+        "d2dx_ddp_multi_work_size": (i64, [i32, i32, i32]),
+        "d2dx_ddp_multi_solve": (C.c_int, [H, P(CollocProblem), i32, P(dbl), P(dbl), c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, P(DdpOptions), c_dp]),
         "d2dx_pursuit_control": (C.c_int, [H, P(Pursuit), i32, c_dp, c_dp, c_dp, c_dp]),
         "d2dx_rollout_pursuit": (C.c_int, [H, P(Pursuit), i32, c_dp, c_dp, c_dp, dbl, i32, i32, i32, c_dp, c_dp, c_dp, c_dp, c_dp]),
         "d2dx_dfma_burn": (C.c_int, [H, i32, i32, i32, c_dp, c_dp]),

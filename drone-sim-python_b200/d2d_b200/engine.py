@@ -334,6 +334,17 @@ class Engine:
                                  C.byref(opts) if opts is not None else None, self.stream_ptr()), "d2dx_ddp_solve")
         self.launches += 1
 
+    def ddp_multi_solve(self, prob, P, bounds, state_box, p0, p1, u, xs, info, lam=None, opts=None):
+        """coupled multi-aircraft solve (one warp per problem): u (P,2,n_ac,N) in/out, xs (P,3,n_ac,N) out, info (P,8) out,
+        lam (P,3,n_ac) out or None, p0 / p1 (P,3,n_ac): device tensors; bounds / state_box host tuples."""
+        b = (C.c_double * 4)(*bounds)
+        sb = (C.c_double * 5)(*state_box) if state_box is not None else None
+        work = self.empty(int(lib.d2dx_ddp_multi_work_size(P, prob.n_ac, prob.N)))
+        check(lib.d2dx_ddp_multi_solve(self.h, C.byref(prob), P, b, sb, _ptr(p0), _ptr(p1), _ptr(u), _ptr(xs), _ptr(info),
+                                       _ptr(lam), _ptr(work), C.byref(opts) if opts is not None else None,
+                                       self.stream_ptr()), "d2dx_ddp_multi_solve")
+        self.launches += 1
+
     # ---- pure pursuit ------------------------------------------------------------------------------------
     def pursuit(self, pts, lookahead=100, K=1., sat_phi=np.deg2rad(45.), v_sp=10.):
         """device copy of a sampled path (n_pts, 2) + the controller constants -> (struct, keep-alive tensors)"""

@@ -91,14 +91,15 @@ def implement_controller(n_ac, time, x_ref, y_ref, v, w, X0s, nsub=10):
     return X, U, Xr, Yd, Ydd, dX
 
 
-def trajectory_optimization(scen, n_starts=1):
-    """Phase 2.1 (11_full_sim_case1.py:180-194) without the plots: returns the solved planner."""
+def trajectory_optimization(scen, n_starts=1, method="auto"):
+    """Phase 2.1 (11_full_sim_case1.py:180-194) without the plots: returns the solved planner.  `method` goes to
+    MultiPlanner.run ("ddp": the coupled second-order solver)."""
     _p = None
     for _case in range(scen.ncases):
         scen.set_case(_case)
         _p = MultiPlanner(scen, initialize=True)
         _p.configure(tol=scen.tol, max_iter=scen.max_iter)
-        _p.run(initial_guess=_p.get_initial_guess(scen.initial_guess), n_starts=n_starts)
+        _p.run(initial_guess=_p.get_initial_guess(scen.initial_guess), n_starts=n_starts, method=method)
         _p.interpret_solution()
     return _p
 
@@ -123,16 +124,18 @@ def ExtendTraj_symm(n_ac, x_ref, y_ref, psi_ref, time):
 def full_sim(df, n_ac=4, v=15, w=(0, 0), r=60, c=((0, -20), (25, -20), (25, -100), (0, -100)),
              X1_f=((0, 40, 0, 0, 12), (25, 40, 0, 0, 12), (25, -40, 0, 0, 12), (0, -40, 0, 0, 12)),
              X2_f=((75, 40, 0, 0, 12), (100, 40, 0, 0, 12), (100, -40, 0, 0, 12), (75, -40, 0, 0, 12)),
-             t_opt=6, t_sim_end=200, t_step=0.05, t_end_1=1000, stop="states", scen=trap_4, n_starts=1):
+             t_opt=6, t_sim_end=200, t_step=0.05, t_end_1=1000, stop="states", scen=trap_4, n_starts=1,
+             method="auto"):
     """main() of 11_full_sim_case1.py:405-499 (stop="states") / 12_full_sim_case2.py (stop="e_theta") without plots.
     `df`: the phase-3 formation trajectory (columns time, x_i, y_i, psi_i; `inf_traj_10s.csv` upstream).
+    `method`: the planner's solver in phase 2 (MultiPlanner.run).
     Returns a dict: X, U, time (all phases appended as upstream), the per-phase pieces and the solved planner."""
     X1, U1, _, _, Ur, e_theta, time_1, t1_f = CircularFormationGVF(np.asarray(c, float), r, v, n_ac, X1_f, 0, t_step, t_end_1, stop=stop)
     X_array, U_array, time = X1, U1, time_1
     # phase 2: plan from the reached states, then track the plan
     X2_i = tuple(map(tuple, X1[-1]))
     scen.t1, scen.p0s, scen.p1s = t_opt, X2_i, X2_f
-    _p = trajectory_optimization(scen, n_starts=n_starts)
+    _p = trajectory_optimization(scen, n_starts=n_starts, method=method)
     x_ref_2, y_ref_2, time_opt = np.array(_p.sol_x).T, np.array(_p.sol_y).T, np.array(_p.sol_time)
     X2, U2, Xr2, Yd2, Ydd2, dX2 = implement_controller(n_ac, time_opt, x_ref_2, y_ref_2, v, list(w), X2_i)
     X_array, U_array = np.append(X_array, X2, axis=0), np.append(U_array, U2, axis=0)

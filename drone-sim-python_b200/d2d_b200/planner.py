@@ -86,6 +86,15 @@ class _PlannerBase:
             info["nfev"] = info["iterations"]
             if method == "auto" and not np.isin(info["flag"], (2, 4)).any():
                 frees = info = None                                   # no start converged: hand the problem to the first-order driver
+        elif method == "ddp":
+            # coupled second-order solve (one GPU warp per start): the caller's start, its mirror image (the other turn directions)
+            # and the perturbed starts drawn above, n_starts in all (at least the first two)
+            k = max(n_starts, 2)
+            phi_s, v_s = np.concatenate([phi[:1], -phi[:1], phi[1:]])[:k], np.concatenate([v[:1], v[:1], v[1:]])[:k]
+            nlp = shooting.ShootingNLP(self.prob, p0, p1, phi_b, v_b, P=len(phi_s), state_box=box)
+            k_enough = (min_solved if min_solved is not None else (3 if n_starts == 1 else 0))
+            frees, info = shooting.solve_ddp(nlp, phi_s, v_s, ctol=min(tol, 1e-6), verbose=verbose, min_solved=k_enough)
+            info["nfev"] = info["iterations"]
         if frees is None:
             nlp = shooting.ShootingNLP(self.prob, p0, p1, phi_b, v_b, P=n_starts, state_box=box)
             driver = shooting.solve_host if _.get("driver") == "host" else shooting.solve

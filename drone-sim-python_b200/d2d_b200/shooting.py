@@ -213,30 +213,43 @@ def solve(nlp, theta, ctol=1e-8, gtol=1e-10, ftol=1e-10, max_outer=30, max_inner
 
 
 def solve_ddp(nlp, phi0, v0, ctol=1e-8, retries=4, opts=None, verbose=False, min_solved=0):
-    """Second-order solve of P single-aircraft problems (d2dx_ddp_solve: control-limited DDP on the collocation grid, one GPU
-    thread per problem).  phi0, v0: host (P, N) (or broadcastable) start inputs.  Problems that end unsolved climb a retry
-    ladder: the same start with the other regularisation (eigenvalue-modified Newton: better on tightly saturated problems,
-    plain Levenberg-Marquardt: better elsewhere), then the mirrored bank profile (the other turn direction -- the usual reason
-    for an infeasible local minimum) with either, and last the original start with four times the sweep budget (the clipped
-    exponential obstacles of exp_4 converge in ~500 sweeps, beyond the default 400).  `min_solved=k` (multi-start of ONE problem): the launch ends as soon as k starts
-    have converged and the ladder is only climbed when none has.  Returns (frees (P, num_free) in the planner layout, info)."""
-    if nlp.n_ac != 1:
-        raise ValueError("solve_ddp handles one aircraft per problem (collision terms couple the aircraft: use solve)")
-    e, P, N = nlp.eng, nlp.P, nlp.N
+    """Second-order solve of P problems: control-limited DDP on the collocation grid.  One aircraft per problem: d2dx_ddp_solve
+    (one GPU thread per problem); several (n_ac <= 10): d2dx_ddp_multi_solve (the aircraft coupled through the collision term,
+    one warp per problem).  phi0, v0: host (P, n_ac, N) start inputs or anything that broadcasts to it ((P, N) when n_ac = 1).
+    Problems that end unsolved climb a retry ladder.  One aircraft: the same start with the other regularisation
+    (eigenvalue-modified Newton: better on tightly saturated problems, plain Levenberg-Marquardt: better elsewhere), then the
+    mirrored bank profile (the other turn direction -- the usual reason for an infeasible local minimum) with either, and last
+    the original start with four times the sweep budget (the clipped exponential obstacles of exp_4 converge in ~500 sweeps,
+    beyond the default 400).  Several aircraft (plain regularisation only): every bank profile mirrored, then the original start
+    with four times the sweep budget.  `min_solved=k` (multi-start of ONE problem): the launch ends as soon as k starts
+    have converged and the ladder is only climbed when none has.  Returns (frees (P, num_free) in the planner layout, info);
+    with several aircraft info["lam"] (P, 3, n_ac) holds the terminal multipliers of each returned solution."""
+    e, P, N, n = nlp.eng, nlp.P, nlp.N, nlp.n_ac
     kw = dict(ctol=ctol, min_solved=int(min_solved)) if opts is None else {f: getattr(opts, f) for f, _ in opts._fields_}
     lo, hi, vlo, vhi = nlp.bounds
-    u0 = np.stack([np.broadcast_to(np.asarray(phi0, np.float64).reshape(-1, N) if np.ndim(phi0) else np.full((1, N), float(phi0)), (P, N)),
-                   np.broadcast_to(np.asarray(v0, np.float64).reshape(-1, N) if np.ndim(v0) else np.full((1, N), float(v0)), (P, N))], 1)
-    u0 = np.clip(u0, np.array([lo, vlo])[None, :, None], np.array([hi, vhi])[None, :, None])
+
+    def starts(a):
+        a = np.asarray(a, np.float64)
+        return np.broadcast_to(a.reshape(-1, 1, N) if n == 1 and a.ndim else a, (P, n, N))
+    u0 = np.clip(np.stack([starts(phi0), starts(v0)], 1), np.array([lo, vlo])[None, :, None, None], np.array([hi, vhi])[None, :, None, None])
     u = e.to_device(np.ascontiguousarray(u0))
-    xs, info = e.empty(P, 3, N), e.zeros(P, 8)
-    p0, p1 = nlp.p0.reshape(P, 3).contiguous(), nlp.p1.reshape(P, 3).contiguous()
+    xs, info, lam = e.empty(P, 3, n, N), e.zeros(P, 8), e.zeros(P, 3, n)
+    p0, p1 = nlp.p0.contiguous(), nlp.p1.contiguous()
+
+    def run(cnt, p0_, p1_, u_, xs_, info_, lam_, o):
+        if n == 1:
+            e.ddp_solve(nlp.c_prob, cnt, nlp.bounds, nlp.state_box, p0_, p1_, u_, xs_, info_, o)
+        else:
+            e.ddp_multi_solve(nlp.c_prob, cnt, nlp.bounds, nlp.state_box, p0_, p1_, u_, xs_, info_, lam_, o)
     mode0 = int(kw.get("reg_mode", 0))
-    e.ddp_solve(nlp.c_prob, P, nlp.bounds, nlp.state_box, p0, p1, u, xs, info, e.ddp_options(**{**kw, "reg_mode": mode0}))
+    run(P, p0, p1, u, xs, info, lam, e.ddp_options(**{**kw, "reg_mode": mode0}))
     ih = info.cpu().numpy()
     total_its = ih[:, 1].copy()
     base = e.ddp_options(**kw)
-    ladder = [(1.0, 1 - mode0, 1), (-1.0, mode0, 1), (-1.0, 1 - mode0, 1), (1.0, mode0, 4)][:retries]
+    if n == 1:
+        ladder = [(1.0, 1 - mode0, 1), (-1.0, mode0, 1), (-1.0, 1 - mode0, 1), (1.0, mode0, 4)][:retries]
+    else:
+        ladder = [(-1.0, mode0, 1), (1.0, mode0, 4)][:retries]
     for r, (sign, mode, scale) in enumerate(ladder):
         bad = np.nonzero(ih[:, 0] != 2)[0]
         if len(bad) == 0 or (min_solved > 0 and len(bad) < P):
@@ -246,18 +259,21 @@ def solve_ddp(nlp, phi0, v0, ctol=1e-8, retries=4, opts=None, verbose=False, min
         if sign < 0 and not np.any(seed[:, 0]):
             seed[:, 0] = 0.3 * hi
         idx = torch.from_numpy(bad).to(e.device)
-        ub, xb, ib = e.to_device(np.ascontiguousarray(seed)), e.empty(len(bad), 3, N), e.zeros(len(bad), 8)
-        e.ddp_solve(nlp.c_prob, len(bad), nlp.bounds, nlp.state_box, p0[idx].contiguous(), p1[idx].contiguous(), ub, xb, ib,
-                    e.ddp_options(**{**kw, "reg_mode": mode, "max_iter": int(base.max_iter) * scale, "max_outer": int(base.max_outer) * (2 if scale > 1 else 1)}))
+        ub, xb, ib, lb = e.to_device(np.ascontiguousarray(seed)), e.empty(len(bad), 3, n, N), e.zeros(len(bad), 8), e.zeros(len(bad), 3, n)
+        run(len(bad), p0[idx].contiguous(), p1[idx].contiguous(), ub, xb, ib, lb,
+            e.ddp_options(**{**kw, "reg_mode": mode, "max_iter": int(base.max_iter) * scale, "max_outer": int(base.max_outer) * (2 if scale > 1 else 1)}))
         ibh = ib.cpu().numpy()
         better = torch.from_numpy((ibh[:, 0] == 2) | (ibh[:, 4] < ih[bad, 4])).to(e.device)
         sel = idx[better]
-        u[sel], xs[sel], info[sel] = ub[better], xb[better], ib[better]
+        u[sel], xs[sel], info[sel], lam[sel] = ub[better], xb[better], ib[better], lb[better]
         total_its[bad] += ibh[:, 1]
         ih = info.cpu().numpy()
         if verbose:
             print(f"retry {r} (bank sign {sign:+.0f}, regularisation {mode}, sweep budget x{scale}): {len(bad)} problems re-seeded, {(ibh[:, 0] == 2).sum()} of them solved")
-    frees = torch.cat([xs.reshape(P, 3 * N), u.reshape(P, 2 * N)], dim=1).cpu().numpy()
-    nlp.xs.copy_(xs.reshape(P, 3, 1, N)); nlp.u_phys.copy_(u.reshape(P, 2, 1, N))
-    return frees, {"flag": ih[:, 0].astype(int), "iterations_each": total_its.astype(int), "iterations": int(total_its.max()), "outer": int(ih[:, 2].max()),
-                   "cost": ih[:, 3].copy(), "c_max": ih[:, 4].copy(), "method": "ddp"}
+    frees = torch.cat([xs.permute(0, 2, 1, 3).reshape(P, 3 * n * N), u.reshape(P, 2 * n * N)], dim=1).cpu().numpy()
+    nlp.xs.copy_(xs); nlp.u_phys.copy_(u)
+    out = {"flag": ih[:, 0].astype(int), "iterations_each": total_its.astype(int), "iterations": int(total_its.max()), "outer": int(ih[:, 2].max()),
+           "cost": ih[:, 3].copy(), "c_max": ih[:, 4].copy(), "method": "ddp"}
+    if n > 1:
+        out["lam"], out["rho"] = lam.cpu().numpy(), ih[:, 7].copy()
+    return frees, out

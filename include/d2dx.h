@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define D2DX_VERSION 104
+#define D2DX_VERSION 105
 
 enum { D2DX_OK = 0, D2DX_EINVAL = 1, D2DX_ECUDA = 2, D2DX_EUNSUPPORTED = 3 };
 
@@ -436,6 +436,23 @@ int64_t d2dx_ddp_work_size(int32_t P, int32_t N);
 int d2dx_ddp_solve(d2dx_handle* h, const d2dx_colloc_problem* p_host, int32_t P, const double* bounds_host4,
                    const double* state_box_host5, const double* p0, const double* p1, double* u, double* xs, double* info,
                    double* work, const d2dx_ddp_options* o_host, void* stream);
+
+/* -------- second-order solve of the multi-aircraft planner NLP (replaces prob.solve -> IPOPT, 07_multioptyplan.py:80-88) --------
+ * The control-limited DDP of d2dx_ddp_solve with the n_ac aircraft of a problem in one stage: 3 n_ac states, 2 n_ac inputs, the
+ * transition block-diagonal per aircraft, the aircraft coupled through the collision term (its exact Hessian in the value model);
+ * the 2 n_ac-variable box QP of every node by projected Newton; 3 n_ac terminal conditions by an augmented Lagrangian.  One WARP
+ * solves one problem.  p_host: 1 <= n_ac <= 10; the cost terms are those of d2dx_shoot_adjoint (soft box on every aircraft,
+ * obstacles on aircraft 0, collision on the pair (0, 1) or every pair).  Layouts as the shooting kernels:
+ *   p0[P][3][n_ac], p1[P][3][n_ac]     initial states and terminal targets (x, y, psi)
+ *   u[P][2][n_ac][N]                   in: start (phi, v), out: solution      xs[P][3][n_ac][N]  out: states of the solution
+ *   info[P][8]                         as d2dx_ddp_solve
+ *   lam_out[P][3][n_ac] or NULL        multipliers of the last inner loop (the returned inputs minimise the Lagrangian for them)
+ *   work                               device doubles, at least d2dx_ddp_multi_work_size(P, n_ac, N)
+ * Options as d2dx_ddp_solve; reg_mode 1 is refused for n_ac > 1 (D2DX_EINVAL), as are n_ac outside 1 .. 10 and bad bounds. */
+int64_t d2dx_ddp_multi_work_size(int32_t P, int32_t n_ac, int32_t N);
+int d2dx_ddp_multi_solve(d2dx_handle* h, const d2dx_colloc_problem* p_host, int32_t P, const double* bounds_host4,
+                         const double* state_box_host5, const double* p0, const double* p1, double* u, double* xs, double* info,
+                         double* lam_out, double* work, const d2dx_ddp_options* o_host, void* stream);
 
 /* -------- pure-pursuit guidance on a sampled path (PurePursuitControler, d2d/guidance.py:204-245; SURVEY 8f #4) --------
  * nearest sample of the path to the aircraft (first minimum of the Euclidean distance, as np.argmin), carrot `lookahead`
