@@ -177,6 +177,8 @@ __global__ void math_probe_kernel(int n, const double* __restrict__ x, const dou
   const double ax = fabs(x[i]), ys = fm::rsqrt_seed(ax);
   out[9 * (size_t)n + i] = fma(-ax * ys, ys, 1.0);
   out[10 * (size_t)n + i] = wrap_pi(x[i]);
+  fm::sincos_small(x[i], s, c);
+  out[11 * (size_t)n + i] = s; out[12 * (size_t)n + i] = c;
 }
 
 }  // namespace d2dx

@@ -316,7 +316,7 @@ __device__ __forceinline__ double turn_rate(double phi, double v) {
   return kG * tn * rcp_f(v * td);
 }
 
-// heading of an RK4 stage by angle addition: sin / cos of psi0 + d from (s0, c0) = sin / cos psi0, |d| < 0.1
+// heading of an RK4 stage by angle addition: sin / cos of psi0 + d from (s0, c0) = sin / cos psi0, |d| < 2^-5
 __device__ __forceinline__ void stage_heading(double s0, double c0, double d, double& s, double& c) {
   double sd, cd;
   fm::sincos_small(d, sd, cd);
@@ -325,14 +325,15 @@ __device__ __forceinline__ void stage_heading(double s0, double c0, double d, do
 }
 
 // |x| below a validity threshold given by its HIGH WORD (integer pipe; NaN compares false).  The thresholds of the fast RK4 path
-// are safety margins, not sharp limits: 0x3FB99999 = just under 0.1, 0x3FF26666 = just under 1.15.
+// are the validity bounds of the small-angle sincos and the tan Pade: 0x3FA00000 = 2^-5, 0x3FF26666 = just under 1.15.  At h = 0.01
+// the 2^-5 bound sends no more steps of the bench workloads to the generic path than a 0.1 bound does (counted: DESIGN 4.1 (f)).
 __device__ __forceinline__ bool abs_below(double x, int thr_hi) { return (__double2hiint(x) & 0x7fffffff) < thr_hi; }
-constexpr int kHiIncr = 0x3FB99999, kHiBank = 0x3FF26666;
+constexpr int kHiIncr = 0x3FA00000, kHiBank = 0x3FF26666;
 
 // Fixed-step stand-in for Aircraft.disc_dyn (d2d/dynamic.py:25-28): nsub classical RK4 sub-steps of cont_dyn
 // (:14-23) with the input held, then psi wrapped once (:27).  Straight-line fast path: the four stage headings share
 // one full sincos (stages 2-4 by angle addition of the increment h psi_dot), tan(phi) is a Pade ratio folded into
-// the 1/v reciprocal.  Validity (|increment| < 0.1, |phi| <= 1.15) is accumulated in one flag; if it is ever violated
+// the 1/v reciprocal.  Validity (|increment| < 2^-5, |phi| <= 1.15) is accumulated in one flag; if it is ever violated
 // the control step is redone with rk4_step_generic.
 // ONE = the caller guarantees nsub == 1 (the Monte-Carlo rollouts): no sub-step loop, so no loop-carried register copies.
 template <bool ONE = false, bool LAG = false>
@@ -341,7 +342,7 @@ __device__ __forceinline__ void rk4_step(const AcPar& a, double* X, double phi_c
   // reciprocal forms differ by at most one ulp of h (1e-16 relative on one step length), far inside the 1e-9 parity bound
   const double h = (ONE || nsub == 1) ? dt : dt * (1.0 / nsub), hh = 0.5 * h, h6 = h * (1.0 / 6.0);
   double x = X[0], y = X[1], psi = X[2], phi = X[3], v = X[4];
-  bool fast_ok = true;                       // every stage increment < 0.1 rad and every bank angle <= 1.15 rad
+  bool fast_ok = true;                       // every stage increment < 2^-5 rad and every bank angle <= 1.15 rad
   const int n_sub = ONE ? 1 : nsub;
 #pragma unroll
   for (int sub = 0; sub < n_sub; ++sub) {

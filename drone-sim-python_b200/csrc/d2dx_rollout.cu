@@ -1,12 +1,14 @@
 // Closed-loop rollout of B aircraft-scenarios under the DFFF controller: one thread = one
 // aircraft-scenario, state in fp64 registers, trajectory parameters staged in shared memory,
 // SoA logs written with coalesced stores.  Replaces run_simulation (05_test_simulation.py:21-34).
+#define D2DX_ATAN_TABLE_IN_SMEM       // the kernel below stages the arctangent knots in its dynamic shared memory
 #include "d2dx_device.cuh"
 #include "d2dx_host.h"
 
 namespace d2dx {
 
 constexpr int kRolloutThreads = 128;
+constexpr size_t kRolloutDynSmem = fm::kAtanTabLen * sizeof(double);     // the arctangent knots (d2dx_math.cuh: atan_knot)
 #ifndef D2DX_ROLLOUT_MIN_BLOCKS
 #define D2DX_ROLLOUT_MIN_BLOCKS 4      // <= 128 registers per thread: 16 resident warps per SM
 #endif
@@ -53,6 +55,8 @@ __global__ void __launch_bounds__(kRolloutThreads, D2DX_ROLLOUT_MIN_BLOCKS) roll
   const int b = active ? b_raw : B - 1;
   const d2dx_traj_table& tt = a.s.traj;
   const int S = tt.n_seg;
+  if (tid < fm::kAtanTabLen) fm::kAtanTabSmem[tid] = fm::kAtanTab[tid];
+  __syncthreads();
 
   // ---- stage the trajectory parameters of this block's scenarios in shared memory ----
   int cur_seg = -1, seg_type = UNIFORM;
@@ -196,16 +200,16 @@ template <int UNIFORM>
 static int launch_rollout(const RolloutArgs& a, bool logging, cudaStream_t st) {
   const int grid = (a.s.B + kRolloutThreads - 1) / kRolloutThreads;
   const bool logref = a.o.Xr_log || a.o.K_log;
-  if (logref) rollout_dfff_kernel<UNIFORM, true, true><<<grid, kRolloutThreads, 0, st>>>(a);
-  else if (logging) rollout_dfff_kernel<UNIFORM, true, false><<<grid, kRolloutThreads, 0, st>>>(a);
-  else rollout_dfff_kernel<UNIFORM, false, false><<<grid, kRolloutThreads, 0, st>>>(a);
+  if (logref) rollout_dfff_kernel<UNIFORM, true, true><<<grid, kRolloutThreads, kRolloutDynSmem, st>>>(a);
+  else if (logging) rollout_dfff_kernel<UNIFORM, true, false><<<grid, kRolloutThreads, kRolloutDynSmem, st>>>(a);
+  else rollout_dfff_kernel<UNIFORM, false, false><<<grid, kRolloutThreads, kRolloutDynSmem, st>>>(a);
   D2DX_LAUNCH_CHECK("rollout_dfff_kernel");
   return D2DX_OK;
 }
 
 int rollout_resident_threads_per_sm() {
   int nb = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rollout_dfff_kernel<D2DX_SEG_CIRCLE, false, false>, kRolloutThreads, 0);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rollout_dfff_kernel<D2DX_SEG_CIRCLE, false, false>, kRolloutThreads, kRolloutDynSmem);
   return nb * kRolloutThreads;
 }
 

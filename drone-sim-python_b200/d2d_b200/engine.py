@@ -366,9 +366,9 @@ class Engine:
         return Xf
 
     def math_probe(self, x, y):
-        """Engine elementary functions on device arrays x, y -> [11][n] (sin, cos, atan2(y,x), atan x, y/x, sqrt|x|, rsqrt|x|, 1/x, and the residuals
-        of the hardware reciprocal and reciprocal-square-root seeds, norm_mpi_pi(x))."""
-        n = x.numel(); out = self.empty(11, n)
+        """Engine elementary functions on device arrays x, y -> [13][n] (sin, cos, atan2(y,x), atan x, y/x, sqrt|x|, rsqrt|x|, 1/x, the residuals
+        of the hardware reciprocal and reciprocal-square-root seeds, norm_mpi_pi(x), and the small-angle sin x, cos x for |x| < 2^-5)."""
+        n = x.numel(); out = self.empty(13, n)
         check(lib.d2dx_math_probe(self.h, n, _ptr(x), _ptr(y), _ptr(out), self.stream_ptr()), "d2dx_math_probe")
         self.launches += 1
         return out

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define D2DX_VERSION 105
+#define D2DX_VERSION 106
 
 enum { D2DX_OK = 0, D2DX_EINVAL = 1, D2DX_ECUDA = 2, D2DX_EUNSUPPORTED = 3 };
 
@@ -480,9 +480,9 @@ int d2dx_rollout_pursuit(d2dx_handle* h, const d2dx_pursuit* p, int32_t B, const
  * thread); the caller times it with CUDA events.  sink: device double[1] (keeps the chains alive). */
 int d2dx_dfma_burn(d2dx_handle* h, int32_t blocks, int32_t threads, int32_t iters, double* sink, void* stream);
 /* the engine's straight-line fp64 elementary functions on n argument pairs (x[n], y[n] device):
- * out[11][n] = sin x, cos x, atan2(y, x), atan x, y / x, sqrt|x|, 1/sqrt|x|, 1/x, and the residuals 1 - x y0, 1 - |x| y0^2 of the
- * hardware reciprocal / reciprocal-square-root seeds the last four start from, and norm_mpi_pi(x) (bit-exact against NumPy's
- * (x + pi) % (2 pi) - pi)   (accuracy tests) */
+ * out[13][n] = sin x, cos x, atan2(y, x), atan x, y / x, sqrt|x|, 1/sqrt|x|, 1/x, and the residuals 1 - x y0, 1 - |x| y0^2 of the
+ * hardware reciprocal / reciprocal-square-root seeds the last four start from, norm_mpi_pi(x) (bit-exact against NumPy's
+ * (x + pi) % (2 pi) - pi), and the small-angle sin x, cos x of the RK4 stage headings (|x| < 2^-5)   (accuracy tests) */
 int d2dx_math_probe(d2dx_handle* h, int32_t n, const double* x, const double* y, double* out, void* stream);
 
 #ifdef __cplusplus
